@@ -5,7 +5,7 @@ features, 512^2 x 400 CT; % HBM peak).
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                   [--workload extract|hist|slab] [--mask ones|lung] [--arith fma|plain]
                   [--rois N] [--no-box] [--overlap] [--no-e2e] [--no-cpu-baseline]
-                  [--no-hist] [--no-slab] [--slab-size S] [--slab-steps K]
+                  [--no-hist] [--no-slab] [--slab-size S] [--slab-steps K] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic scan: ImageToEmphysemaFeaturesFilter
 semantics (masked normalized convolution -> gradient magnitude -> fused Hessian/eigen
@@ -31,7 +31,23 @@ Prints ONE JSON line (rank 0).  `value` is device-resident throughput (CUDA even
 launching stream, max over ranks); `e2e` goes through the C ABI with pinned HOST buffers, H2D
 and D2H inside the timed region; `roofline` is the dominant kernel's algorithmic bytes / its
 measured launch time against MEASURED_PEAKS.json; `cpu_baseline` is the CPU oracle timed on
-this box's host cores on a bounded sample of the same workload.
+this box's host cores on a bounded sample of the same workload.  Every timed loop runs
+--steps K steps (the slab leg: --slab-steps when given; a step of the hist leg's batch
+sub-legs is one call of 8 scans).
+
+--dump-outputs DIR (rank 0) writes, right after each leg's timed steps, what its last step
+returned to the caller, so that two builds can be compared output for output on the same
+seeded inputs:
+  extract_features.npy        float32 (n_sigma, 8, DUMP_VOXELS)  the feature volumes at
+                              DUMP_VOXELS voxel positions drawn with a fixed seed
+  hist_edges.npy              float32 (n_sigma*8, 40)  the edges the hist leg bins with (derived
+                              from the scan's features by the library under test)
+  hist_whole_mask_counts.npy  float64 (1, n_sigma*8, 41)
+  hist_rois_counts.npy        float64 (min(rois, DUMP_ROIS), n_sigma*8, 41)  the first ROIs' counts
+  slab_features.npy           float32 (scales in the last call, 8, DUMP_VOXELS) of rank 0's slab
+  slab_edges.npy              float32 (n_sigma*8, 40)  like hist_edges, from the first 64 planes
+  slab_counts.npy             float64 (n_sigma*8, 41)
+At most 2 x 4 x 8 x DUMP_VOXELS x 4 B = 32 MB of samples plus 11 MB of counts.
 """
 import argparse
 import json
@@ -43,6 +59,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True       # the benchmark writes nothing into the (possibly read-only) tree
 sys.path.insert(0, os.path.join(ROOT, "image-feature-extraction_b200"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -61,6 +78,8 @@ CPU_SAMPLE_NZ = 64                   # CPU arms (cpu_baseline, --impl reference)
 CPU_SAMPLE = "%dx%dx%d sub-volume x %d scales" % (DIMS[0], DIMS[1], CPU_SAMPLE_NZ, len(SIGMAS))
 HIST_SAMPLE_Z0 = 32                  # hist parity sample: planes [32, 96) -- the lung mask starts at z = 50
 N_EDGES = 40
+DUMP_VOXELS = 1 << 17                # --dump-outputs: voxel positions sampled from each feature stack
+DUMP_ROIS = 1000                     # --dump-outputs: ROI histograms written at most
 WORKLOAD = ("ExtractFeatures multi-scale eigen features (8 masked feature volumes per scale) on one "
             "512x512x400 float CT-like scan per GPU, sigma{0.6,1.2,2.4,4.8}; the CPU arms (cpu_baseline, "
             "--impl reference) time a bounded sample of it per step: " + CPU_SAMPLE)
@@ -70,7 +89,7 @@ def measured_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
         return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    return 6553.3, "B200 device-copy bandwidth of BASELINE.md (no MEASURED_PEAKS.json)"
 
 
 def traffic_for(workload, kernel):
@@ -460,6 +479,29 @@ def kernel_table(env, prof, algo, voxels_per_launch, ms_total, workload_key):
     return table
 
 
+def dump_output(env, name, arr):
+    """--dump-outputs: DIR/<name>.npy from rank 0.  arr: numpy, or a device tensor of counts."""
+    if not env.args.dump_outputs or env.rank != 0:
+        return
+    import numpy as np
+    if not isinstance(arr, np.ndarray):
+        arr = arr.to(env.torch.float64).cpu().numpy()
+    os.makedirs(env.args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(env.args.dump_outputs, name + ".npy"), arr)
+
+
+def dump_feature_sample(env, name, feats):
+    """--dump-outputs: (S, 8, nz, ny, nx) device features -> (S, 8, DUMP_VOXELS) float32 at voxel
+    positions drawn with a fixed seed (the same positions for every build and run)."""
+    if not env.args.dump_outputs or env.rank != 0:
+        return
+    import numpy as np
+    nvox = feats[0, 0].numel()
+    idx = np.sort(np.random.default_rng(0).choice(nvox, size=min(DUMP_VOXELS, nvox), replace=False))
+    pick = env.torch.from_numpy(idx).to(feats.device)
+    dump_output(env, name, feats.reshape(feats.shape[:2] + (nvox,))[:, :, pick].cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------
 # headline leg: ExtractFeatures semantics, one scan per GPU
 # ------------------------------------------------------------------------------------------
@@ -476,6 +518,7 @@ def leg_extract(env, img, mask):
         ctx.emphysema_features_dev(img.data_ptr(), mask.data_ptr(), out.data_ptr(), DIMS, SIGMAS)
 
     ms, launches, prof, clocks = env.timed(step, args.steps, env.warmup, clocks=True)
+    dump_feature_sample(env, "extract_features", out)     # before the other arithmetic mode overwrites `out`
     ms_per_step = ms / args.steps
     value = env.world * units / (ms_per_step * 1e-3) / 1e9
     wd = ctx.last_work_dims()
@@ -501,12 +544,11 @@ def leg_extract(env, img, mask):
         alt = env.ife.ARITH_PLAIN if args.arith == "fma" else env.ife.ARITH_FMA
         ctx.set_arith(alt)
         try:
-            ms_o, _, _, _ = env.timed(step, max(3, min(args.steps, 5)), 2, clocks=False)
+            ms_o, _, _, _ = env.timed(step, args.steps, 2, clocks=False)
         finally:
             ctx.set_arith(env.ife.ARITH_FMA if args.arith == "fma" else env.ife.ARITH_PLAIN)
-        n_o = max(3, min(args.steps, 5))
-        other = {"arith": "plain" if args.arith == "fma" else "fma", "ms_per_step": ms_o / n_o,
-                 "value": units / (ms_o / n_o * 1e-3) / 1e9, "unit": "Gvoxel/s",
+        other = {"arith": "plain" if args.arith == "fma" else "fma", "ms_per_step": ms_o / args.steps,
+                 "value": units / (ms_o / args.steps * 1e-3) / 1e9, "unit": "Gvoxel/s",
                  "note": "same workload, device-resident, the recursion's other arithmetic mode (bit-exact against the oracle in that mode)"}
     e2e = None
     if not args.no_e2e:
@@ -522,7 +564,7 @@ def leg_extract(env, img, mask):
             ctx._check(ctx.L.ife_cuda_emphysema_features(ctx.h, C.c_void_p(h_img.data_ptr()), C.c_void_p(h_mask.data_ptr()),
                                                          C.c_void_p(h_out.data_ptr()), dims_c, sp_c, sig_c, len(SIGMAS),
                                                          env.ife.MEM_HOST))
-        e_steps = max(1, min(args.steps, 5))
+        e_steps = args.steps
         for _ in range(2):
             e2e_step()
         env.barrier()
@@ -630,6 +672,10 @@ def leg_hist(env, mask_kind="lung", n_rois=50, headline=False):
     # invariant at full size: every row of the whole-mask histogram holds every in-mask voxel once
     row_sums = counts[0].to(torch.int64).sum(1)
     res["whole_mask"]["row_sums_equal_mask_voxels"] = bool((row_sums == int(mask_np.sum())).all().item())
+    dump_output(env, "hist_edges", edges)
+    dump_output(env, "hist_whole_mask_counts", counts)
+    if n_rois > 0:
+        dump_output(env, "hist_rois_counts", counts_r[:DUMP_ROIS])
 
     if not args.no_e2e:
         h_img = torch.empty((nz, ny, nx), dtype=torch.float32, pin_memory=True).copy_(img)
@@ -642,7 +688,7 @@ def leg_hist(env, mask_kind="lung", n_rois=50, headline=False):
             ctx._check(ctx.L.ife_cuda_emphysema_histograms(ctx.h, C.c_void_p(h_img.data_ptr()), C.c_void_p(h_mask.data_ptr()),
                                                            dims_c, sp_c, sig_c, len(SIGMAS), edges.ctypes.data_as(C.c_void_p),
                                                            N_EDGES, None, 0, h_counts.ctypes.data_as(C.c_void_p), env.ife.MEM_HOST))
-        e_steps = max(1, min(args.steps, 5))
+        e_steps = args.steps
         for _ in range(2):
             e2e_step()
         env.barrier()
@@ -661,10 +707,11 @@ def leg_hist(env, mask_kind="lung", n_rois=50, headline=False):
         ctx.emphysema_histograms_batch(imgs, masks, SIGMAS, edges, None)
         env.barrier()
         t0 = time.perf_counter()
-        ctx.emphysema_histograms_batch(imgs, masks, SIGMAS, edges, None)
-        dtb = env.max_over_ranks((time.perf_counter() - t0) / nb)
+        for _ in range(args.steps):       # one step = one call of nb scans
+            ctx.emphysema_histograms_batch(imgs, masks, SIGMAS, edges, None)
+        dtb = env.max_over_ranks((time.perf_counter() - t0) / (nb * args.steps))
         e2e["batch"] = {"value": env.world * units / dtb / 1e9, "unit": "Gvoxel/s", "ms_per_scan": dtb * 1e3,
-                        "scans_per_call": nb, "api": "ife_cuda_emphysema_histograms_batch (host scans, uploads overlapped)"}
+                        "scans_per_call": nb, "steps": args.steps, "api": "ife_cuda_emphysema_histograms_batch (host scans, uploads overlapped)"}
         # the same batch with the scans as int16 on the host (CT's type on disk; option
         # "host_image_i16": 2 bytes per voxel up, widened on the device) -- the synthetic scan is
         # rounded to integers for this sub-leg, so its histograms are those of the rounded scan
@@ -675,12 +722,13 @@ def leg_hist(env, mask_kind="lung", n_rois=50, headline=False):
             ctx.emphysema_histograms_batch(imgs16, masks, SIGMAS, edges, None, _raw_image=True)
             env.barrier()
             t0 = time.perf_counter()
-            ctx.emphysema_histograms_batch(imgs16, masks, SIGMAS, edges, None, _raw_image=True)
-            dt16 = env.max_over_ranks((time.perf_counter() - t0) / nb)
+            for _ in range(args.steps):
+                ctx.emphysema_histograms_batch(imgs16, masks, SIGMAS, edges, None, _raw_image=True)
+            dt16 = env.max_over_ranks((time.perf_counter() - t0) / (nb * args.steps))
         finally:
             ctx.set_option("host_image_i16", 0)
         e2e["batch_int16_upload"] = {"value": env.world * units / dt16 / 1e9, "unit": "Gvoxel/s", "ms_per_scan": dt16 * 1e3,
-                                     "scans_per_call": nb, "h2d_bytes_per_scan": int(h_i16.numel() * 2 + h_mask.numel()),
+                                     "scans_per_call": nb, "steps": args.steps, "h2d_bytes_per_scan": int(h_i16.numel() * 2 + h_mask.numel()),
                                      "api": "ife_cuda_emphysema_histograms_batch, option host_image_i16"}
         res["e2e"] = e2e
         del h_img, h_mask, h_i16
@@ -725,7 +773,7 @@ def leg_slab(env):
     z0, z1 = ife.slab_range(size, world, rank)
     nzo = z1 - z0
     n_own = nzo * plane
-    steps = args.slab_steps
+    steps = args.slab_steps or args.steps
     # every rank builds the whole volume: its own planes feed the slab path, all of them the
     # single-GPU reference of the parity block
     full = synth_volume_torch(torch, dev, 4, (size, size, size), z_range=(0, size))
@@ -761,6 +809,9 @@ def leg_slab(env):
                                             edges=edges, counts_ptr=counts.data_ptr(), halo_factor=halo_factor)
 
     ms, launches, prof, clocks = env.timed(run_once, steps, env.warmup, clocks=True)
+    dump_feature_sample(env, "slab_features", out)        # before the parity block reuses `out`
+    dump_output(env, "slab_edges", edges)
+    dump_output(env, "slab_counts", counts)
     ms_per_step = ms / steps
     units = size ** 3 * len(SIGMAS)
     value = units / (ms_per_step * 1e-3) / 1e9
@@ -856,7 +907,7 @@ def _main(out_stream):
     ap.add_argument("--mask", default="ones", choices=["ones", "lung"])
     ap.add_argument("--arith", default="fma", choices=["fma", "plain"])
     ap.add_argument("--slab-size", type=int, default=1024)
-    ap.add_argument("--slab-steps", type=int, default=10)
+    ap.add_argument("--slab-steps", type=int, default=None, help="slab leg: timed steps (default: --steps)")
     ap.add_argument("--halo-factor", type=float, default=12.0)
     ap.add_argument("--rois", type=int, default=50, help="hist leg: bin into N fixed-seed 41^3 ROIs (MakeBag) besides the whole mask")
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -866,7 +917,12 @@ def _main(out_stream):
     ap.add_argument("--no-slab-parity", action="store_true")
     ap.add_argument("--no-box", action="store_true", help="A/B: smooth the whole volume even where the mask cannot see it")
     ap.add_argument("--overlap", action="store_true", help="option overlap_scales: features of scale s beside the passes of scale s+1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what each leg's last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or (args.slab_steps is not None and args.slab_steps < 1):
+        ap.error("--steps and --slab-steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference has none")
     if args.impl == "reference":
         if "--steps" not in " ".join(sys.argv):
             args.steps = 3                   # ~4 s of CPU work per step
