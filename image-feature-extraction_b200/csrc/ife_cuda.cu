@@ -26,6 +26,7 @@
 #include "recursive_gaussian.cuh"
 #include "iir_tma.cuh"
 #include "radix_sort.cuh"
+#include "resample.cuh"
 #include "support_box.cuh"
 #include "ife_ctx.h"
 
@@ -1725,6 +1726,79 @@ int ife_cuda_intensity_roi_histograms(ife_cuda_ctx* ctx, const float* image, con
   if (mem == IFE_MEM_HOST) {
     IFE_CUDA_TRY(ctx, cudaMemcpyAsync(counts, d_counts, n_counts * sizeof(uint32_t),
                                       cudaMemcpyDeviceToHost, ctx->stream()));
+    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
+  }
+  return IFE_OK;
+}
+
+int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_bytes, const int dims[3],
+                      const double spacing[3], const double out_spacing[3], int interp, double default_value,
+                      int out_dims[3], int mem) {
+  if (!ctx && out) return IFE_E_INVALID;   // a size query needs no context (nor a device)
+  if (!in || !out_dims || !out_spacing) return fail(ctx, IFE_E_INVALID, "null pointer argument");
+  if (interp != IFE_INTERP_LINEAR && interp != IFE_INTERP_NEAREST)
+    return fail(ctx, IFE_E_INVALID, "unknown interpolator %d", interp);
+  if (elem_bytes != 4 && elem_bytes != 1) return fail(ctx, IFE_E_INVALID, "elem_bytes must be 4 (float) or 1 (uint8)");
+  if (interp == IFE_INTERP_LINEAR && elem_bytes != 4)
+    return fail(ctx, IFE_E_INVALID, "linear interpolation takes float voxels only");
+  if (elem_bytes == 1 && !(default_value >= 0.0 && default_value <= 255.0 && default_value == std::floor(default_value)))
+    return fail(ctx, IFE_E_INVALID, "default value %g is not a uint8 value", default_value);
+  IFE_TRY(check_dims(ctx, dims, spacing));
+  int m[3];
+  for (int d = 0; d < 3; ++d) {
+    if (!std::isfinite(spacing[d])) return fail(ctx, IFE_E_INVALID, "spacing[%d] is not finite", d);
+    if (!(out_spacing[d] > 0.0) || !std::isfinite(out_spacing[d]))
+      return fail(ctx, IFE_E_INVALID, "out_spacing[%d] = %g must be positive and finite", d, out_spacing[d]);
+    // n' = max(1, floor(n * s / s' + 0.5)), in double
+    const double want = std::floor((double)dims[d] * spacing[d] / out_spacing[d] + 0.5);
+    if (!(want <= 2147483647.0)) return fail(ctx, IFE_E_INVALID, "output axis %d would have %g voxels", d, want);
+    m[d] = std::max(1, (int)want);
+  }
+  const size_t n_in = (size_t)dims[0] * dims[1] * dims[2], n_out = (size_t)m[0] * m[1] * m[2];
+  if (m[1] > 65535 * kRsBY || m[2] > 65535) return fail(ctx, IFE_E_INVALID, "output grid %d x %d x %d is too large", m[0], m[1], m[2]);
+  for (int d = 0; d < 3; ++d) out_dims[d] = m[d];
+  if (!out) return IFE_OK;
+  IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const uint8_t* d_in;
+  IFE_TRY(stage_in(ctx, ctx->ws.in_img, static_cast<const uint8_t*>(in), n_in * elem_bytes, mem, &d_in));
+  void* d_out = out;
+  if (mem == IFE_MEM_HOST) {
+    IFE_TRY(ctx->ws.out[0].reserve(ctx, n_out * elem_bytes));
+    d_out = ctx->ws.out[0].ptr;
+  }
+  ResampleArgs A;
+  std::memset(&A, 0, sizeof(A));
+  A.in = d_in;
+  A.out = d_out;
+  for (int d = 0; d < 3; ++d) {
+    A.n[d] = dims[d];
+    A.m[d] = m[d];
+    A.so[d] = out_spacing[d];
+    A.inv[d] = 1.0 / spacing[d];
+    A.ident[d] = out_spacing[d] == spacing[d];
+  }
+  A.def_f32 = (float)default_value;
+  A.def_u8 = elem_bytes == 1 ? (uint8_t)default_value : 0;
+  const int mode = interp == IFE_INTERP_LINEAR ? RS_LINEAR : elem_bytes == 4 ? RS_NEAREST_F32 : RS_NEAREST_U8;
+  const bool vec = m[0] % kRsV == 0 && reinterpret_cast<uintptr_t>(d_out) % (kRsV * elem_bytes) == 0;
+  const dim3 block(kRsBX, kRsBY), grid((unsigned)((m[0] + kRsBX * kRsV - 1) / (kRsBX * kRsV)),
+                                       (unsigned)((m[1] + kRsBY - 1) / kRsBY), (unsigned)m[2]);
+  {
+    ProfScope prof(ctx, K_OTHER);
+    cudaStream_t st = ctx->stream();
+    switch (mode * 2 + (vec ? 1 : 0)) {
+      case 0: resample_kernel<RS_LINEAR, false><<<grid, block, 0, st>>>(A); break;
+      case 1: resample_kernel<RS_LINEAR, true><<<grid, block, 0, st>>>(A); break;
+      case 2: resample_kernel<RS_NEAREST_F32, false><<<grid, block, 0, st>>>(A); break;
+      case 3: resample_kernel<RS_NEAREST_F32, true><<<grid, block, 0, st>>>(A); break;
+      case 4: resample_kernel<RS_NEAREST_U8, false><<<grid, block, 0, st>>>(A); break;
+      default: resample_kernel<RS_NEAREST_U8, true><<<grid, block, 0, st>>>(A); break;
+    }
+    ctx->launches++;
+    IFE_CUDA_TRY(ctx, cudaGetLastError());
+  }
+  if (mem == IFE_MEM_HOST) {
+    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, n_out * elem_bytes, cudaMemcpyDeviceToHost, ctx->stream()));
     IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
   }
   return IFE_OK;

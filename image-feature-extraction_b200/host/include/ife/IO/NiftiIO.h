@@ -292,7 +292,21 @@ template <typename T>
 void Write(const std::string& path, const Geometry& g, const T* data) {
   ScopedSeconds clock(write_seconds());
   std::vector<unsigned char> hdr(352, 0);
-  if (g.nifti_header.size() == 348) std::copy(g.nifti_header.begin(), g.nifti_header.end(), hdr.begin());
+  if (g.nifti_header.size() == 348) {
+    std::copy(g.nifti_header.begin(), g.nifti_header.end(), hdr.begin());
+    // a spacing that differs from the one Read() took from the header (resampling) replaces pixdim
+    // and scales the sform's column of that axis; the qform takes its scale from pixdim itself
+    for (int d = 0; d < 3; ++d) {
+      const double p = std::fabs((double)rd<float>(hdr, 76 + 4 * (d + 1), false));
+      const double was = p > 0 ? p : 1.0;
+      if (g.spacing[d] == was) continue;
+      wr<float>(hdr, 76 + 4 * (d + 1), (float)g.spacing[d]);
+      for (int r = 0; r < 3; ++r) {
+        const size_t off = 280 + 16 * r + 4 * d;   // srow_x / srow_y / srow_z, column d
+        wr<float>(hdr, off, (float)(rd<float>(hdr, off, false) * (g.spacing[d] / was)));
+      }
+    }
+  }
   wr<int32_t>(hdr, 0, 348);
   int16_t dim[8] = {3, (int16_t)g.size[0], (int16_t)g.size[1], (int16_t)g.size[2], 1, 1, 1, 1};
   std::memcpy(hdr.data() + 40, dim, sizeof(dim));

@@ -2,7 +2,8 @@
 // (ValueArg / MultiArg with a short flag, a long name, a required bit and a default):
 // `-i path`, `--image path`, `--image=path`, repeated flags for MultiArg, `-h/--help`,
 // `--version`.  Parse errors print "PARSE ERROR" with the offending argument and make the
-// tool exit with EXIT_FAILURE, as TCLAP's default handler does.
+// tool exit with EXIT_FAILURE, as TCLAP's default handler does.  An argument with nargs > 1
+// takes that many values after its flag (`-s 0.7 0.7 2.5`).
 #ifndef IFE_B200_CMDLINE_H
 #define IFE_B200_CMDLINE_H
 #include <cstdlib>
@@ -20,6 +21,7 @@ public:
     bool required, multi;
     std::vector<std::string> values;
     bool set = false;
+    int nargs = 1;
   };
   CmdLine(const std::string& message, const std::string& version) : m_Message(message), m_Version(version) {}
 
@@ -62,6 +64,10 @@ public:
       if (arg->set && !arg->multi) return error("Argument already set!", tok, exit_code);
       if (!arg->multi) arg->values.clear();
       arg->values.push_back(val);
+      for (int k = 1; k < arg->nargs; ++k) {
+        if (i + 1 >= argc) return error("This argument takes " + std::to_string(arg->nargs) + " values!", tok, exit_code);
+        arg->values.push_back(argv[++i]);
+      }
       arg->set = true;
     }
     for (const Arg& a : m_Args)
@@ -91,7 +97,8 @@ public:
   void usage(std::ostream& os) const {
     os << "USAGE:" << std::endl << "   " << m_Prog;
     for (const Arg& a : m_Args) {
-      const std::string one = "-" + a.flag + " <" + a.type + ">";
+      std::string one = "-" + a.flag;
+      for (int k = 0; k < a.nargs; ++k) one += " <" + a.type + ">";
       os << " " << (a.required ? one : "[" + one + "]") << (a.multi ? " ..." : "");
     }
     os << " [--version] [-h]" << std::endl << std::endl << "Where:" << std::endl;

@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("IFE_CUDA_LIB") or os.path.join(_HERE, "lib", "libife_
 HEADER_PATH = os.path.normpath(os.path.join(_HERE, "..", "include", "ife_cuda.h"))
 
 MEM_HOST, MEM_DEVICE = 0, 1
+INTERP_LINEAR, INTERP_NEAREST = 0, 1
 ARITH_PLAIN, ARITH_FMA = 0, 1
 FDHF_TOOL_DY_BUG = 1
 NUM_FEATURES = 8
@@ -76,6 +77,7 @@ def load_library():
     L.ife_cuda_intensity_roi_histograms.argtypes = [vp, vp, vp, ip, vp, i, vp, i, vp, i]
     L.ife_cuda_eigen_features_batch.argtypes = [vp, vp, vp, sz, i]
     L.ife_cuda_sort_f32.argtypes = [vp, vp, sz, i]
+    L.ife_cuda_resample.argtypes = [vp, vp, vp, i, ip, dp, dp, i, d, ip, i]
     L.ife_cuda_emphysema_feature_samples.argtypes = [vp, vp, vp, vp, vp, sz, ip, dp, dp, i, i, vp, C.POINTER(sz), i]
     L.ife_cuda_host_alloc.argtypes = [sz, C.POINTER(C.c_void_p)]
     L.ife_cuda_host_free.argtypes = [vp]
@@ -109,6 +111,14 @@ def slab_range(nz, n_ranks, rank):
 def slab_halo(sigma, spacing_z=1.0, halo_factor=12.0):
     import math
     return int(math.ceil(halo_factor * sigma / spacing_z)) + 5
+
+
+def resampled_dims(dims, spacing, out_spacing):
+    """(nx, ny, nz) of ife_cuda_resample's output grid: max(1, floor(n * s / s' + 0.5)) per axis in
+    double, the library's rule (pure host arithmetic, for sizing device buffers)."""
+    import math
+    return tuple(max(1, int(math.floor(int(n) * float(s) / float(so) + 0.5)))
+                 for n, s, so in zip(dims, spacing, out_spacing))
 
 
 def _i3(dims):
@@ -347,6 +357,20 @@ class Context:
             self._check(self.L.ife_cuda_emphysema_feature_samples(*args, _ptr(out), C.byref(n_out), MEM_HOST))
         return out
 
+    def resample(self, vol, spacing, out_spacing, nearest=False, default=0.0):
+        """(nz, ny, nx) float32 or uint8 volume at voxel spacing (sx, sy, sz) -> the volume resampled
+        to out_spacing (linear: float32 only; nearest: float32 or uint8, the type is kept)."""
+        vol = np.ascontiguousarray(vol)
+        if vol.dtype not in (np.float32, np.uint8):
+            raise TypeError("resample takes float32 or uint8 volumes, not %s" % vol.dtype)
+        od = (C.c_int * 3)()
+        args = (_i3(_dims_of(vol)), _d3(spacing), _d3(out_spacing), INTERP_NEAREST if nearest else INTERP_LINEAR,
+                float(default), od, MEM_HOST)
+        self._check(self.L.ife_cuda_resample(self.h, _ptr(vol), None, vol.dtype.itemsize, *args))  # sizes only
+        out = np.empty((od[2], od[1], od[0]), vol.dtype)
+        self._check(self.L.ife_cuda_resample(self.h, _ptr(vol), _ptr(out), vol.dtype.itemsize, *args))
+        return out
+
     def eigen_features_batch(self, A6):
         A6 = np.ascontiguousarray(A6, np.float32).reshape(-1, 6)
         out = np.empty_like(A6)
@@ -378,6 +402,16 @@ class Context:
     def normalized_gaussian_dev(self, img_ptr, cert_f32_ptr, out_ptr, dims, sigma, spacing=None, mask_output=False):
         self._check(self.L.ife_cuda_normalized_gaussian(self.h, _ptr(img_ptr), _ptr(cert_f32_ptr), None, _ptr(out_ptr),
                                                         _i3(dims), _d3(spacing), sigma, int(mask_output), MEM_DEVICE))
+
+    def resample_dev(self, in_ptr, out_ptr, dims, spacing, out_spacing, elem_bytes=4, nearest=False,
+                     default=0.0):
+        """Device-pointer resample (enqueued on the context's stream) -> out_dims (nx, ny, nz);
+        out_ptr=None only computes out_dims."""
+        od = (C.c_int * 3)()
+        self._check(self.L.ife_cuda_resample(
+            self.h, _ptr(in_ptr), _ptr(out_ptr), elem_bytes, _i3(dims), _d3(spacing), _d3(out_spacing),
+            INTERP_NEAREST if nearest else INTERP_LINEAR, float(default), od, MEM_DEVICE))
+        return tuple(int(v) for v in od)
 
     def hessian_eigen_features_dev(self, img_ptr, mask_ptr, out_ptr, dims, sigma, spacing=None,
                                    flags=0):

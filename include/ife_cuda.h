@@ -245,6 +245,27 @@ int ife_cuda_intensity_roi_histograms(ife_cuda_ctx* ctx, const float* image, con
                                       const int dims[3], const float* edges, int n_edges,
                                       const int* rois, int n_roi, uint32_t* counts, int mem);
 
+/* Resampling onto a new voxel spacing: itk::ResampleImageFilter with an identity transform and the
+ * output origin equal to the input's (the reference's Resample tool, which is not part of the port
+ * otherwise; DESIGN.md "Resampling" restates the semantics and lists where they differ from ITK).
+ *   out_dims[d] = max(1, floor(dims[d] * spacing[d] / out_spacing[d] + 0.5)) in double; out_dims is
+ *   always written, and out == NULL only queries it (in must still be given; ctx may then be NULL,
+ *   so the query works without a device);
+ *   continuous index c = (i * out_spacing[d]) * (1 / spacing[d]), c = i where the spacings are equal;
+ *   outside -0.5 <= c < dims[d] - 0.5 on any axis the voxel is default_value;
+ *   IFE_INTERP_LINEAR: LinearInterpolateImageFunction, float voxels only (elem_bytes 4).
+ *     PRECONDITION: the input is finite (a zero-weight Inf or NaN neighbour would poison the lerp);
+ *   IFE_INTERP_NEAREST: NearestNeighborInterpolateImageFunction, index floor(c + 0.5); float or uint8
+ *     voxels (elem_bytes 4 or 1; for uint8 default_value must be an integer in [0, 255]).
+ * in and out have the layout and `mem` of every volume of this ABI (x fastest, dims = {nx,ny,nz}).
+ * IFE_E_INVALID for a null in, a non-positive or non-finite spacing, linear with elem_bytes 1, or an
+ * unknown interp. */
+#define IFE_INTERP_LINEAR 0
+#define IFE_INTERP_NEAREST 1
+int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_bytes,
+                      const int dims[3], const double spacing[3], const double out_spacing[3],
+                      int interp, double default_value, int out_dims[3], int mem);
+
 /* Ascending in-place sort of n floats: the `std::sort` of the feature samples in
  * tools/DetermineHistogramBinEdges_MultiScaleEigenvalueFeatures.cxx:282-283.  A radix sort of
  * this library's own (csrc/radix_sort.cuh: 4-bit digits, count / scan / stable scatter; no
