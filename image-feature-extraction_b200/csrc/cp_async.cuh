@@ -1,4 +1,4 @@
-// cp.async (LDGSTS) helpers shared by the Gaussian passes and the fused feature kernel.
+// cp.async (LDGSTS) helpers of the fused feature kernels.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -7,26 +7,12 @@ namespace ife {
 __device__ __forceinline__ void cp_async4(void* smem, const void* gmem) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem));
 }
-__device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem));
-}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem));
-}
-
-// 16-byte copy whose line is marked evict-first in L2: the last use of streamed data
-__device__ __forceinline__ unsigned long long l2_evict_first_policy() {
-  unsigned long long pol;
-  asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void cp_async16_hint(void* smem, const void* gmem, unsigned long long pol) {
-  asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"((unsigned)__cvta_generic_to_shared(smem)),
-               "l"(gmem), "l"(pol));
 }
 
 }  // namespace ife

@@ -66,11 +66,9 @@ struct ife_cuda_ctx {
   cudaEvent_t events[4] = {nullptr, nullptr, nullptr, nullptr};
   cudaEvent_t ov_events[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // overlap_scales: input ready, blur[0..1] written, blur[0..1] consumed
   uint64_t launches = 0;
-  bool use_async = true;   // cp.async software-pipelined Gaussian passes (option "async_passes")
   bool use_tma = true;     // tensor-map staged, field-per-warp Gaussian passes where the layout allows (option "tma_passes")
   bool use_march4 = true;  // fused feature kernel with four voxels per thread where the layout allows (option "march4")
   bool host_image_i16 = false;   // host image pointers of the ife_cuda_emphysema_* calls are int16 (option "host_image_i16")
-  bool tma_balance = false;// tensor-map passes: run one or two blocks per SM fewer when that saves a round (option "tma_balance")
   bool use_box = true;     // masked paths smooth only the mask's support box (option "support_box")
   int* box_host = nullptr; // pinned: the mask extents come back here once per call
   bool overlap_scales = false;   // option "overlap_scales": features of scale s run beside the passes of scale s+1

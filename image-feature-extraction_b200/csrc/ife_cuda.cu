@@ -169,21 +169,13 @@ StencilCoef make_stencil_coef(const double spacing[3]) {
 // Recursive Gaussian passes
 // ---------------------------------------------------------------------------------------
 constexpr int kChunk = 16;
-#ifndef IFE_CHUNK_S
-#define IFE_CHUNK_S 16     // chunk length of the pipelined strided (y / z) passes
-#endif
-#ifndef IFE_MINB_S
-#define IFE_MINB_S 3
-#endif
-constexpr int kChunkS = IFE_CHUNK_S;
 #ifndef IFE_XWARPS
 #define IFE_XWARPS 4
 #endif
 constexpr int kXWarps = IFE_XWARPS;
 
 size_t ckpt_bytes(int nf, int n, size_t n_lines) {
-  constexpr int kc = kChunkS < kChunk ? kChunkS : kChunk;
-  const int n_chunks = (n + kc - 1) / kc;
+  const int n_chunks = (n + kChunk - 1) / kChunk;
   return (size_t)std::max(n_chunks - 1, 0) * nf * 4 * n_lines * sizeof(double);
 }
 
@@ -248,31 +240,6 @@ int make_map3(ife_cuda_ctx* ctx, CUtensorMap* m, const void* base, bool u8, long
 #define IFE_TMA_MINB_X 8
 #endif
 
-// How many blocks per SM a tensor-map pass should run with: the largest count the kernel's own
-// resources allow (`fit`), or one or two fewer when that needs fewer rounds per resident block
-// (cost model: rounds x blocks per SM, the passes being throughput-bound).  Measured: the model does
-// not hold -- z 10 vs 11: 0.562 / 0.563 ms, y 11 vs 12: 0.586 / 0.578, x 7 vs 8: 0.546 / 0.560 -- latency
-// hiding matters as much as the last round, so the option "tma_balance" is off by default.  IFE_TMA_BLOCKS_{Z,Y,X}
-// in the environment overrides (experiments).  0 = leave the request alone.
-int tma_blocks_per_sm(const ife_cuda_ctx* ctx, int axis, long long blocks, int smem_need) {
-  static const char* names[3] = {"IFE_TMA_BLOCKS_Z", "IFE_TMA_BLOCKS_Y", "IFE_TMA_BLOCKS_X"};
-  if (const char* e = std::getenv(names[axis])) return std::atoi(e);
-  // the x pass (three staging slots per warp, TMA-latency-sensitive) is measurably faster with
-  // seven blocks per SM than with the eight its shared memory allows: 0.544 vs 0.555 ms
-  if (axis == AX_X && !ctx->tma_balance) return 233472 / (smem_need + 1024) > 7 ? 7 : 0;
-  if (!ctx->tma_balance) return 0;
-  const int fit = std::min(axis == AX_X ? IFE_TMA_MINB_X : (axis == AX_Z ? IFE_TMA_MINB_Z : IFE_TMA_MINB_S),
-                           233472 / (smem_need + 1024));
-  int best = fit;
-  long long best_cost = -1;
-  for (int b = fit; b >= std::max(1, fit - 2); --b) {
-    const long long slots = (long long)b * ctx->sm_count;
-    const long long cost = ((blocks + slots - 1) / slots) * b;
-    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = b; }
-  }
-  return best == fit ? 0 : best;
-}
-
 template <int AXIS, int INMODE, bool DIVIDE, int MASKMODE = 0>
 int launch_tma_pass(ife_cuda_ctx* ctx, const GaussCoef& C, const CUtensorMap& i0, const CUtensorMap& i1,
                     const CUtensorMap& o0, const CUtensorMap& o1, const TmaArgs& A, dim3 grid) {
@@ -281,11 +248,12 @@ int launch_tma_pass(ife_cuda_ctx* ctx, const GaussCoef& C, const CUtensorMap& i0
   constexpr size_t smem_need = (INMODE == IN_IMG_U8    ? kRegionImgU8 + kRegionU8 + kOnesTile
                                 : INMODE == IN_IMG_F32 ? kRegionImgF32 + kRegionF32 + kOnesTile
                                                        : 2 * (AXIS == AX_X ? kRegionX : kRegionF32)) + kTmaBarBytes;
-  // Blocks per SM: all blocks of a pass take the same time, so the pass costs ceil(blocks / slots)
-  // rounds.  Where one block per SM fewer turns a nearly empty last round into a full one, the
-  // shared memory request is padded so that exactly `want` blocks fit (tma_blocks_per_sm()).
-  const int want = tma_blocks_per_sm(ctx, AXIS, (long long)grid.x * grid.y, (int)smem_need);
-  const size_t smem = want > 0 ? std::max<size_t>(smem_need, (size_t)(233472 / want - 1024) / 128 * 128) : smem_need;
+  // The x pass (three staging slots per warp, TMA-latency-sensitive) is measurably faster with seven
+  // blocks per SM than with the eight its shared memory allows (0.544 vs 0.555 ms): where more than
+  // seven would fit (233472 B per SM, 1 KB of it reserved per block), the shared-memory request is
+  // padded so that exactly seven do.
+  constexpr bool seven = AXIS == AX_X && 233472 / (smem_need + 1024) > 7;
+  constexpr size_t smem = seven ? std::max<size_t>(smem_need, (233472 / 7 - 1024) / 128 * 128) : smem_need;
   if (ctx->arith == IFE_ARITH_FMA) {
     auto kern = iir_tma_kernel<AXIS, INMODE, DIVIDE, true, MINB, MASKMODE>;
     IFE_CUDA_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -319,66 +287,16 @@ bool tma_gaussian_usable(const ife_cuda_ctx* ctx, const float* in0, const void* 
   return al(in0) && al(out0) && encode_tiled_fn() != nullptr;
 }
 
-constexpr int kAsyncStages = 3;
-
-template <int NF, int INMODE, bool DIVIDE, int MASKMODE, bool FMA>
-int launch_strided_async_m(ife_cuda_ctx* ctx, const GaussCoef& C, const PassArgs& A) {
-  // Measured (512x512x400, two fields): the y pass (float fields, divide sink) is fastest with
-  // the replay buffer in shared memory, 2 stages and 3 CTAs/SM (0.91 vs 0.99 ms); the z pass
-  // (uint8 mask input) with the replay buffer in registers, 3 stages, 2 CTAs/SM (0.67 vs 0.71).
-  constexpr bool YBS = NF == 2;
-  constexpr int STAGES = YBS ? 2 : kAsyncStages;
-  constexpr int MINB = YBS ? IFE_MINB_S : 1;
-  auto kern = gauss_pass_strided_async<NF, INMODE, DIVIDE, MASKMODE, kChunkS, FMA, STAGES, YBS, MINB>;
-  const size_t smem = sizeof(AsyncStage<NF, INMODE, kChunkS, !YBS>) * STAGES +
-                      (YBS ? (size_t)NF * kChunkS * kAsyncThreads * sizeof(double) : 0);
-  IFE_CUDA_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const unsigned grid = (unsigned)((A.n_lines + kAsyncThreads - 1) / kAsyncThreads);
-  kern<<<grid, kAsyncThreads, smem, ctx->stream()>>>(C, A);
-  return IFE_OK;
-}
-
-template <int NF, int INMODE, bool DIVIDE, bool FMA>
-int launch_strided_async(ife_cuda_ctx* ctx, const GaussCoef& C, const PassArgs& A) {
-  if (DIVIDE && A.mask_u8) return launch_strided_async_m<NF, INMODE, DIVIDE, DIVIDE ? 1 : 0, FMA>(ctx, C, A);
-  if (DIVIDE && A.mask_f32) return launch_strided_async_m<NF, INMODE, DIVIDE, DIVIDE ? 2 : 0, FMA>(ctx, C, A);
-  return launch_strided_async_m<NF, INMODE, DIVIDE, 0, FMA>(ctx, C, A);
-}
-
 template <int NF, int INMODE, bool DIVIDE>
 int launch_strided(ife_cuda_ctx* ctx, const GaussCoef& C, const PassArgs& A) {
   const unsigned grid = (unsigned)((A.n_lines + 127) / 128);
   ProfScope prof(ctx, A.stride == (long long)A.na && A.sb == 0 ? K_PASS_Z : K_PASS_Y);
-  // software-pipelined kernel when every warp's 32 lines are contiguous and 16-byte aligned
-  const bool contiguous = A.sb == 0 || A.na % 32 == 0;   // no warp straddles two line groups
-  bool async_ok = ctx->use_async && contiguous && A.n_lines % 4 == 0 && A.stride % 4 == 0 &&
-                  (A.sb % 4 == 0) && reinterpret_cast<uintptr_t>(A.in0) % 16 == 0 &&
-                  (NF == 1 || reinterpret_cast<uintptr_t>(A.in1) % 16 == 0);
-  if (INMODE == IN_IMG_U8) async_ok = async_ok && A.stride % 16 == 0 && A.n_lines % 16 == 0;
-  if (async_ok) {
-    if (ctx->arith == IFE_ARITH_FMA) IFE_TRY((launch_strided_async<NF, INMODE, DIVIDE, true>(ctx, C, A)));
-    else IFE_TRY((launch_strided_async<NF, INMODE, DIVIDE, false>(ctx, C, A)));
-  } else if (ctx->arith == IFE_ARITH_FMA) {
+  if (ctx->arith == IFE_ARITH_FMA)
     gauss_pass_strided<NF, INMODE, DIVIDE, kChunk, true><<<grid, 128, 0, ctx->stream()>>>(C, A);
-  } else {
+  else
     gauss_pass_strided<NF, INMODE, DIVIDE, kChunk, false><<<grid, 128, 0, ctx->stream()>>>(C, A);
-  }
   ctx->launches++;
   IFE_CUDA_TRY(ctx, cudaGetLastError());
-  return IFE_OK;
-}
-
-template <int NF, bool FMA>
-int launch_x_async(ife_cuda_ctx* ctx, const GaussCoef& C, const PassArgs& A) {
-#ifndef IFE_X_STAGES
-#define IFE_X_STAGES kAsyncStages
-#endif
-  auto kern = gauss_pass_x_async<NF, kChunk, FMA, kXWarps, IFE_X_STAGES>;
-  const size_t smem = kXWarps * (IFE_X_STAGES * sizeof(XStage<NF, kChunk>) + sizeof(XOut<NF, kChunk>));
-  IFE_CUDA_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long lines_per_block = 32LL * kXWarps;
-  const unsigned grid = (unsigned)((A.n_lines + lines_per_block - 1) / lines_per_block);
-  kern<<<grid, 32 * kXWarps, smem, ctx->stream()>>>(C, A);
   return IFE_OK;
 }
 
@@ -387,18 +305,10 @@ int launch_x(ife_cuda_ctx* ctx, const GaussCoef& C, const PassArgs& A) {
   const long long lines_per_block = 32LL * kXWarps;
   const unsigned grid = (unsigned)((A.n_lines + lines_per_block - 1) / lines_per_block);
   ProfScope prof(ctx, K_PASS_X);
-  const bool async_ok = ctx->use_async && A.n % 4 == 0 && reinterpret_cast<uintptr_t>(A.in0) % 16 == 0 &&
-                        reinterpret_cast<uintptr_t>(A.out0) % 16 == 0 &&
-                        (NF == 1 || (reinterpret_cast<uintptr_t>(A.in1) % 16 == 0 &&
-                                     reinterpret_cast<uintptr_t>(A.out1) % 16 == 0));
-  if (async_ok) {
-    if (ctx->arith == IFE_ARITH_FMA) IFE_TRY((launch_x_async<NF, true>(ctx, C, A)));
-    else IFE_TRY((launch_x_async<NF, false>(ctx, C, A)));
-  } else if (ctx->arith == IFE_ARITH_FMA) {
+  if (ctx->arith == IFE_ARITH_FMA)
     gauss_pass_x<NF, kChunk, true, kXWarps><<<grid, 32 * kXWarps, 0, ctx->stream()>>>(C, A);
-  } else {
+  else
     gauss_pass_x<NF, kChunk, false, kXWarps><<<grid, 32 * kXWarps, 0, ctx->stream()>>>(C, A);
-  }
   ctx->launches++;
   IFE_CUDA_TRY(ctx, cudaGetLastError());
   return IFE_OK;
@@ -552,6 +462,8 @@ int smooth_volume(ife_cuda_ctx* ctx, const float* in0, const void* cert, bool ce
     return IFE_OK;
   }
 
+  // Plain register-staged kernels (any layout): the same lines as above, each swept whole; the
+  // samples outside the windows that they also write are never read.
   PassArgs A;
   std::memset(&A, 0, sizeof(A));
   A.ckpt = (double*)ws.ckpt.ptr;
@@ -559,7 +471,6 @@ int smooth_volume(ife_cuda_ctx* ctx, const float* in0, const void* cert, bool ce
   // z pass: lines = nx*ny columns, contiguous across the plane
   A.in0 = in0; A.in1 = cert; A.out0 = a0; A.out1 = a1;
   A.n = nzb; A.stride = (long long)nx * ny; A.na = nx * ny > 0 ? nx * ny : 1; A.sb = 0;
-  A.out_lo = kz0; A.out_hi = kz1;   // a z-slab's halo planes only carry recursion state
   A.n_lines = (long long)nx * ny;
   if (nf == 1) IFE_TRY((launch_strided<1, IN_FIELDS, false>(ctx, cz, A)));
   else if (cert_is_u8) IFE_TRY((launch_strided<2, IN_IMG_U8, false>(ctx, cz, A)));
@@ -572,7 +483,6 @@ int smooth_volume(ife_cuda_ctx* ctx, const float* in0, const void* cert, bool ce
   const size_t koff = (size_t)kz0 * plane, boff = (size_t)(kz0 - keep0) * plane;
   A.in0 = a0 + koff; A.in1 = a1 + koff; A.out0 = b0 + boff; A.out1 = b1 + boff;
   A.n = nx; A.stride = 1; A.na = 1; A.sb = 0; A.n_lines = (long long)ny * nzk;
-  A.out_lo = 0; A.out_hi = nx;
   if (nf == 1) IFE_TRY((launch_x<1>(ctx, cx, A)));
   else IFE_TRY((launch_x<2>(ctx, cx, A)));
 
@@ -580,7 +490,6 @@ int smooth_volume(ife_cuda_ctx* ctx, const float* in0, const void* cert, bool ce
   const size_t yoff = boff + (size_t)kx0;
   A.in0 = b0 + yoff; A.in1 = b1 + yoff; A.out0 = out0 + yoff; A.out1 = nullptr;
   A.n = ny; A.stride = nx; A.na = kx1 - kx0; A.sb = (long long)plane; A.n_lines = (long long)(kx1 - kx0) * nzk;
-  A.out_lo = ky0; A.out_hi = ky1;
   A.mask_u8 = outmask_u8 ? outmask_u8 + yoff : nullptr;
   A.mask_f32 = outmask_f32 ? outmask_f32 + yoff : nullptr;
   if (nf == 1) IFE_TRY((launch_strided<1, IN_FIELDS, false>(ctx, cy, A)));
@@ -1156,10 +1065,8 @@ int ife_cuda_last_work_dims(const ife_cuda_ctx* ctx, int dims[3]) {
 
 int ife_cuda_set_option(ife_cuda_ctx* ctx, const char* name, int value) {
   if (!ctx || !name) return IFE_E_INVALID;
-  if (std::strcmp(name, "async_passes") == 0) { ctx->use_async = value != 0; return IFE_OK; }
   if (std::strcmp(name, "tma_passes") == 0) { ctx->use_tma = value != 0; return IFE_OK; }
   if (std::strcmp(name, "march4") == 0) { ctx->use_march4 = value != 0; return IFE_OK; }
-  if (std::strcmp(name, "tma_balance") == 0) { ctx->tma_balance = value != 0; return IFE_OK; }
   if (std::strcmp(name, "host_image_i16") == 0) { ctx->host_image_i16 = value != 0; return IFE_OK; }
   if (std::strcmp(name, "support_box") == 0) { ctx->use_box = value != 0; return IFE_OK; }
   if (std::strcmp(name, "overlap_scales") == 0) { ctx->overlap_scales = value != 0; return IFE_OK; }

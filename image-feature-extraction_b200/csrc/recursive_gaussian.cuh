@@ -31,10 +31,6 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
-#include "cp_async.cuh"
-#ifndef IFE_CACHE_HINTS
-#define IFE_CACHE_HINTS 0
-#endif
 #include "fdiv.cuh"
 
 namespace ife {
@@ -131,31 +127,10 @@ __device__ __forceinline__ size_t ckpt_index(int chunk, int f, int k, size_t n_l
 // the recurrence.  GENERIC = true handles the first chunk (boundary coefficients), the
 // last chunk(s) and partial chunks.
 // ---------------------------------------------------------------------------------------
-// EDGE (hot path only, GENERIC = false): bit 0 = the chunk starts the line (its first four
-// causal samples take the boundary coefficients, chosen at compile time), bit 1 = the chunk
-// ends the line (likewise its last four anticausal samples).  The chunk must be full.
-template <int NF, int L, bool FMA, bool GENERIC, int UNROLL = L, int EDGE = 0, typename SRC>
+template <int NF, int L, bool FMA, bool GENERIC, int UNROLL = L, typename SRC>
 __device__ __forceinline__ void forward_chunk(const GaussCoef& C, const SRC& src, int i0, int len,
                                               Rec (&cs)[NF]) {
   Fb fb = fb_select(C.D, C.BN, 4);
-  if (!GENERIC && (EDGE & 1)) {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const Fb fe = fb_select(C.D, C.BN, j);
-      double v[NF];
-      src(j, v);
-#pragma unroll
-      for (int f = 0; f < NF; ++f) causal_step<FMA>(C, fe, cs[f], v[f]);
-    }
-#pragma unroll UNROLL
-    for (int j = 4; j < L; ++j) {
-      double v[NF];
-      src(j, v);
-#pragma unroll
-      for (int f = 0; f < NF; ++f) causal_step<FMA>(C, fb, cs[f], v[f]);
-    }
-    return;
-  }
 #pragma unroll UNROLL
   for (int j = 0; j < L; ++j) {
     if (!GENERIC || j < len) {
@@ -169,22 +144,15 @@ __device__ __forceinline__ void forward_chunk(const GaussCoef& C, const SRC& src
 }
 
 // Where the replayed causal values of a chunk wait for the anticausal sweep: registers
-// (RegYB) or a per-thread column of shared memory (SmemYB), which frees 4*L registers per
-// thread and lets a third CTA fit on the SM.
+// (RegYB) here, a per-warp buffer in shared memory in the tensor-map kernels (iir_tma.cuh).
 template <int NF, int L>
 struct RegYB {
   double v[NF][L];
   __device__ __forceinline__ void set(int f, int j, double x) { v[f][j] = x; }
   __device__ __forceinline__ double get(int f, int j) const { return v[f][j]; }
 };
-template <int NF, int L, int THREADS>
-struct SmemYB {
-  double* col;  // this thread's column: element (f, j) at col[(f*L + j)*THREADS]
-  __device__ __forceinline__ void set(int f, int j, double x) { col[(f * L + j) * THREADS] = x; }
-  __device__ __forceinline__ double get(int f, int j) const { return col[(f * L + j) * THREADS]; }
-};
 
-template <int NF, int L, bool FMA, bool GENERIC, int UNROLL = L, int EDGE = 0, typename SRC, typename SINK, typename YB>
+template <int NF, int L, bool FMA, bool GENERIC, int UNROLL = L, typename SRC, typename SINK, typename YB>
 __device__ __forceinline__ void backward_chunk(const GaussCoef& C, const SRC& src, const SINK& sink,
                                                int i0, int len, int n, Rec (&cs)[NF],
                                                Rec (&as)[NF], YB& yb) {
@@ -200,28 +168,8 @@ __device__ __forceinline__ void backward_chunk(const GaussCoef& C, const SRC& sr
     const Fb fc = fb_select(C.D, C.BN, 4);
     const Fb fa = fb_select(C.D, C.BM, 4);
     constexpr int U2 = UNROLL >= L ? L / 2 : UNROLL;
-    constexpr int T0 = EDGE != 0 ? 4 : 0;
-    if (EDGE != 0) {
-      // a chunk at the start / end of the line: the four samples that still see the virtual
-      // constant extension sit in the first four steps (causal j = t, anticausal j = L-1-t)
-      static_assert(EDGE == 0 || L / 2 >= 4, "edge steps must fall into the first half");
-#pragma unroll
-      for (int t = 0; t < 4; ++t) {
-        const int jc = t, ja = L - 1 - t;
-        const Fb fce = (EDGE & 1) ? fb_select(C.D, C.BN, t) : fc;
-        const Fb fae = (EDGE & 2) ? fb_select(C.D, C.BM, t) : fa;
-        double vc[NF], va[NF];
-        src(jc, vc);
-        src(ja, va);
-#pragma unroll
-        for (int f = 0; f < NF; ++f) {
-          yb.set(f, jc, causal_step<FMA>(C, fce, cs[f], vc[f]));
-          yb.set(f, ja, anti_step<FMA>(C, fae, as[f], va[f]));
-        }
-      }
-    }
 #pragma unroll U2
-    for (int t = T0; t < L / 2; ++t) {
+    for (int t = 0; t < L / 2; ++t) {
       const int jc = t, ja = L - 1 - t;
       double vc[NF], va[NF];
       src(jc, vc);
@@ -357,9 +305,7 @@ struct PassArgs {
   const float* mask_f32;    //   "
   double* ckpt;
   int n;                // samples per line
-  int out_lo, out_hi;   // samples [out_lo, out_hi) of every line are wanted (z-slabs: the rest
-                        // is warm-up halo); outside it only the recursion state is advanced
-  long long stride;     // element stride between consecutive samples of a line
+  long long stride;    // element stride between consecutive samples of a line
   int na;               // lines are indexed l = a + na*b, base = a + b*sb  (strided pass)
   long long sb;
   long long n_lines;
@@ -500,360 +446,6 @@ gauss_pass_strided(const __grid_constant__ GaussCoef C, const __grid_constant__ 
       }
     }
   }
-}
-
-// ---------------------------------------------------------------------------------------
-// Strided lines, software-pipelined: the same sweep as gauss_pass_strided, but every chunk
-// (its L samples, the 3 samples of causal history before it and, in phase B, its
-// checkpoint) is brought into shared memory with cp.async STAGES-1 chunks ahead of its use.
-// A warp copies exactly the columns its own 32 lines need (see stage_issue), so no block
-// barrier exists anywhere: cp.async.wait_group + __syncwarp order a warp's copies before
-// its reads.  With 2 CTAs of 128 threads per SM and 3 stages, >100 KB per SM is in flight,
-// which is what hides HBM latency at the 8 resident warps the 200+ registers of the
-// recurrence allow.  Alignment requirements are checked on the host (else the plain
-// register-staged kernel runs).
-// ---------------------------------------------------------------------------------------
-constexpr int kAsyncThreads = 128;
-#ifndef IFE_YBS_UNROLL
-#define IFE_YBS_UNROLL 4
-#endif
-constexpr int kYbsUnroll = IFE_YBS_UNROLL;
-// boundary (first / last / partial) chunks of the strided passes: rolled loops; unrolling by the
-// recursion order makes the state rotation free there too
-#ifndef IFE_GEN_UNROLL
-#define IFE_GEN_UNROLL 1
-#endif
-constexpr int kGenUnroll = IFE_GEN_UNROLL;
-// full chunks at the start / end of a line take the interleaved hot loop with compile-time
-// boundary coefficients instead of the rolled generic loops (strided passes, two fields)
-#ifndef IFE_EDGE_HOT
-#define IFE_EDGE_HOT 1
-#endif
-
-template <int NF, int INMODE, int L, bool CK = true>
-struct AsyncStage {
-  static constexpr int ROWS = L + 3;  // rows 0..2 = samples i0-3..i0-1, rows 3.. = the chunk
-  float f0[ROWS][kAsyncThreads];
-  // second field (float) or certainty (float / uint8, the latter packed in the first bytes)
-  float f1[NF == 2 ? ROWS : 1][kAsyncThreads];
-  double ck[CK ? NF * 4 : 1][CK ? kAsyncThreads : 2];   // checkpoint slots (CK) or none
-};
-
-template <int NF, int INMODE, int L, bool CK>
-__device__ __forceinline__ void stage_sample(const AsyncStage<NF, INMODE, L, CK>& S, int row, int t,
-                                             double (&v)[NF]) {
-  if (INMODE == IN_FIELDS) {
-    v[0] = (double)S.f0[row][t];
-    if (NF == 2) v[NF - 1] = (double)S.f1[NF == 2 ? row : 0][t];
-  } else {
-    const float img = S.f0[row][t];
-    float c;
-    if (INMODE == IN_IMG_U8)
-      c = (float)reinterpret_cast<const uint8_t*>(&S.f1[0][0])[row * kAsyncThreads + t];
-    else
-      c = S.f1[NF == 2 ? row : 0][t];
-    v[0] = (double)__fmul_rn(img, c);  // itk::MultiplyImageFilter
-    v[NF - 1] = (double)c;
-  }
-}
-
-
-// Issue the copies of chunk kc (planes i0-3+row_first .. i0+L-1, clipped to the line) into
-// stage S.  Warp-cooperative 16-byte copies: a warp's 32 lines are 128 contiguous bytes per
-// plane, so one cp.async.cg instruction (32 lanes x 16 B) moves 4 planes of a float field
-// (16 planes of the uint8 mask) -- 5 instructions per field per chunk instead of 19 per
-// thread.  The data a thread reads was copied by other lanes of ITS OWN warp, so a
-// __syncwarp after cp.async.wait_group is all the synchronisation needed.
-// Host-checked: every warp's 32 lines are contiguous in memory (line stride 1, no wrap),
-// pointers and plane strides are 16-byte aligned, n_lines % 4 == 0 (% 16 with a uint8 mask).
-template <int NF, int INMODE, int L, bool CK>
-__device__ __forceinline__ void stage_issue(const PassArgs& A, AsyncStage<NF, INMODE, L, CK>& S, int t,
-                                            size_t wbase, long long wline, size_t line, bool active,
-                                            int kc, int row_first, bool with_ckpt) {
-  constexpr int ROWS = L + 3;
-  const int lane = t & 31, wcol = t & ~31;
-  const int i0 = kc * L;
-  const size_t st = (size_t)A.stride;
-  {
-    const int q = lane >> 3, c = lane & 7;              // 4 planes x 8 chunks of 4 floats
-    const bool grp_ok = wline + 4 * c < A.n_lines;
-#pragma unroll
-    for (int m = 0; m < (ROWS + 3) / 4; ++m) {
-      const int r = 4 * m + q;
-      const int plane = i0 - 3 + r;
-      if (r < ROWS && r >= row_first && plane >= 0 && plane < A.n && grp_ok) {
-        const size_t idx = wbase + (size_t)plane * st + 4 * c;
-        cp_async16(&S.f0[r][wcol + 4 * c], A.in0 + idx);
-        if (NF == 2 && INMODE != IN_IMG_U8)
-          cp_async16(&S.f1[NF == 2 ? r : 0][wcol + 4 * c], reinterpret_cast<const float*>(A.in1) + idx);
-      }
-    }
-  }
-  if (NF == 2 && INMODE == IN_IMG_U8) {
-    const int q = lane >> 1, h = lane & 1;              // 16 planes x 2 chunks of 16 bytes
-    const bool grp_ok = wline + 16 * h < A.n_lines;
-    uint8_t* m8 = reinterpret_cast<uint8_t*>(&S.f1[0][0]);
-#pragma unroll
-    for (int m = 0; m < (ROWS + 15) / 16; ++m) {
-      const int r = 16 * m + q;
-      const int plane = i0 - 3 + r;
-      if (r < ROWS && r >= row_first && plane >= 0 && plane < A.n && grp_ok)
-        cp_async16(m8 + r * kAsyncThreads + wcol + 16 * h,
-                   reinterpret_cast<const uint8_t*>(A.in1) + wbase + (size_t)plane * st + 16 * h);
-    }
-  }
-  if (CK && with_ckpt && kc >= 1 && active) {
-    const double* src = A.ckpt + ckpt_index<NF>(kc, 0, 0, A.n_lines, line);
-#pragma unroll
-    for (int k = 0; k < NF * 4; ++k) cp_async8(&S.ck[k][t], src + (size_t)k * (size_t)A.n_lines);
-  }
-  cp_async_commit();
-}
-
-// Interior chunks of fully populated warps: every plane of the chunk exists and every lane's
-// group of lines is valid, so the copies need no predicates and their addresses are one
-// per-lane base pointer plus warp-uniform plane offsets.
-template <int NF, int INMODE, int L, bool CK>
-__device__ __forceinline__ void stage_issue_fast(const PassArgs& A, AsyncStage<NF, INMODE, L, CK>& S, int t,
-                                                 size_t wbase, int kc, int row_first, bool last_use,
-                                                 unsigned long long pol) {
-  constexpr int ROWS = L + 3;
-  const int lane = t & 31, wcol = t & ~31;
-  const size_t st = (size_t)A.stride;
-  const size_t p0 = wbase + (size_t)(kc * L - 3) * st;   // plane of row 0
-  {
-    const int q = lane >> 3, c = lane & 7;
-    const float* g0 = A.in0 + p0 + (size_t)q * st + 4 * c;
-    const float* g1 = reinterpret_cast<const float*>(A.in1) + p0 + (size_t)q * st + 4 * c;
-    float* s0 = &S.f0[q][wcol + 4 * c];
-    float* s1 = &S.f1[NF == 2 ? q : 0][wcol + 4 * c];
-#pragma unroll
-    for (int m = 0; m < (ROWS + 3) / 4; ++m) {
-      if (4 * m + 3 < row_first) continue;                       // uniform: rows 0..2 only in phase B
-      const bool on = (4 * m + 3 < ROWS || 4 * m + q < ROWS) && 4 * m + q >= row_first;
-      if (on) {
-        if (IFE_CACHE_HINTS && last_use) {
-          cp_async16_hint(s0 + 4 * m * kAsyncThreads, g0 + (size_t)(4 * m) * st, pol);
-          if (NF == 2 && INMODE != IN_IMG_U8) cp_async16_hint(s1 + 4 * m * kAsyncThreads, g1 + (size_t)(4 * m) * st, pol);
-        } else {
-          cp_async16(s0 + 4 * m * kAsyncThreads, g0 + (size_t)(4 * m) * st);
-          if (NF == 2 && INMODE != IN_IMG_U8) cp_async16(s1 + 4 * m * kAsyncThreads, g1 + (size_t)(4 * m) * st);
-        }
-      }
-    }
-  }
-  if (NF == 2 && INMODE == IN_IMG_U8) {
-    const int q = lane >> 1, h = lane & 1;
-    uint8_t* m8 = reinterpret_cast<uint8_t*>(&S.f1[0][0]);
-    const uint8_t* g = reinterpret_cast<const uint8_t*>(A.in1) + p0 + (size_t)q * st + 16 * h;
-#pragma unroll
-    for (int m = 0; m < (ROWS + 15) / 16; ++m) {
-      const int r = 16 * m + q;
-      if (r < ROWS && r >= row_first)
-        cp_async16(m8 + r * kAsyncThreads + wcol + 16 * h, g + (size_t)(16 * m) * st);
-    }
-  }
-  cp_async_commit();
-}
-
-// MASKMODE (DIVIDE only): 0 = no output mask, 1 = uint8 mask, 2 = float mask
-// YBS: the replayed causal values live in shared memory and checkpoints are prefetched into
-// registers instead of stage slots; with STAGES = 2 that is 70 KB per CTA and < 170
-// registers per thread, so three CTAs (12 warps, 6 independent recurrences per SM
-// sub-partition) are resident instead of two.
-template <int NF, int INMODE, bool DIVIDE, int MASKMODE, int L, bool FMA, int STAGES, bool YBS, int MINB>
-__global__ void __launch_bounds__(kAsyncThreads, MINB)
-gauss_pass_strided_async(const __grid_constant__ GaussCoef C, const __grid_constant__ PassArgs A) {
-  using Stage = AsyncStage<NF, INMODE, L, !YBS>;
-  extern __shared__ __align__(16) unsigned char async_smem[];
-  Stage* stages = reinterpret_cast<Stage*>(async_smem);
-  const int t = threadIdx.x;
-  SmemYB<NF, L, kAsyncThreads> ybs{reinterpret_cast<double*>(async_smem + STAGES * sizeof(Stage)) + t};
-  const long long line_ll = (long long)blockIdx.x * kAsyncThreads + t;
-  const bool active = line_ll < A.n_lines;
-  const size_t line = (size_t)(active ? line_ll : A.n_lines - 1);
-  const size_t base = (size_t)(line % A.na) + (size_t)(line / A.na) * (size_t)A.sb;
-  // first line of this warp (its 32 lines are contiguous in memory: host-checked)
-  const long long wline = line_ll - (t & 31);
-  const long long wl = wline < A.n_lines ? wline : A.n_lines - 1;
-  const size_t wbase = (size_t)(wl % A.na) + (size_t)(wl / A.na) * (size_t)A.sb;
-  const size_t st = (size_t)A.stride;
-  const int n = A.n;
-  const int n_chunks = (n + L - 1) / L;
-
-  Rec cs[NF];
-  Rec as[NF];
-
-  // chunks [0, kA) need the causal sweep (nothing above the output range does); chunks
-  // [k_lo, n_chunks) the anticausal one; only chunks in [k_lo, kA) produce output
-  const int kA = min(n_chunks, (A.out_hi + L - 1) / L);
-  const int k_lo = max(0, A.out_lo) / L;
-
-  // copies of chunk kc into a stage: predicate-free for interior chunks of full warps
-  const bool warp_full = wline + 32 <= A.n_lines;
-  const unsigned long long pol = l2_evict_first_policy();
-  auto issue = [&](Stage& S, int kc, int row_first, bool with_ckpt) {
-    if (YBS && warp_full && kc * L - 3 + row_first >= 0 && kc * L + L <= n)
-      stage_issue_fast<NF, INMODE, L, !YBS>(A, S, t, wbase, kc, row_first, with_ckpt, pol);
-    else
-      stage_issue<NF, INMODE, L, !YBS>(A, S, t, wbase, wline, line, active, kc, row_first, with_ckpt);
-  };
-
-  // ---- phase A: causal sweep, checkpoint at every chunk start ----
-#pragma unroll
-  for (int s = 0; s < STAGES - 1; ++s) {
-    if (s < kA) issue(stages[s], s, 3, false);
-    else cp_async_commit();
-  }
-  for (int k = 0; k < kA; ++k) {
-    const int kn = k + STAGES - 1;
-    if (kn < kA) issue(stages[kn % STAGES], kn, 3, false);
-    else cp_async_commit();
-    cp_async_wait<STAGES - 1>();
-    __syncwarp();
-    const Stage& S = stages[k % STAGES];
-    const int i0 = k * L;
-    const int len = min(L, n - i0);
-    if (k == 0) {
-      double v[NF];
-      stage_sample<NF, INMODE, L, !YBS>(S, 3, t, v);
-#pragma unroll
-      for (int f = 0; f < NF; ++f) rec_fill(cs[f], v[f]);
-    } else if (active) {
-#pragma unroll
-      for (int f = 0; f < NF; ++f) {
-        A.ckpt[ckpt_index<NF>(k, f, 0, A.n_lines, line)] = cs[f].h0;
-        A.ckpt[ckpt_index<NF>(k, f, 1, A.n_lines, line)] = cs[f].h1;
-        A.ckpt[ckpt_index<NF>(k, f, 2, A.n_lines, line)] = cs[f].h2;
-        A.ckpt[ckpt_index<NF>(k, f, 3, A.n_lines, line)] = cs[f].h3;
-      }
-    }
-    auto src = [&](int j, double (&v)[NF]) { stage_sample<NF, INMODE, L, !YBS>(S, 3 + j, t, v); };
-    if (len == L && i0 >= 4) forward_chunk<NF, L, FMA, false, YBS ? kYbsUnroll : L>(C, src, i0, len, cs);
-    else if (IFE_EDGE_HOT && YBS && len == L && i0 == 0) forward_chunk<NF, L, FMA, false, kYbsUnroll, 1>(C, src, i0, len, cs);
-    else forward_chunk<NF, L, FMA, true, YBS ? kGenUnroll : L>(C, src, i0, len, cs);
-    if (k == n_chunks - 1) {  // the line's last sample is the anticausal edge value
-      double v[NF];
-      stage_sample<NF, INMODE, L, !YBS>(S, 3 + len - 1, t, v);
-#pragma unroll
-      for (int f = 0; f < NF; ++f) rec_fill(as[f], v[f]);
-    }
-    __syncwarp();  // every lane is done with this stage before any lane refills it
-  }
-  cp_async_wait<0>();
-  __threadfence_block();
-  if (kA < n_chunks) {  // phase A stopped early: fetch the edge value directly
-    float v[NF];
-    load_sample<NF, INMODE>(A, base + (size_t)(n - 1) * st, v);
-#pragma unroll
-    for (int f = 0; f < NF; ++f) rec_fill(as[f], (double)v[f]);
-  }
-
-  // ---- phase B: backward over chunks, prefetching downwards ----
-  double ckn[NF][4];   // YBS: checkpoint of the chunk processed next, prefetched into registers
-  if (YBS) {
-#pragma unroll
-    for (int f = 0; f < NF; ++f)
-#pragma unroll
-      for (int k = 0; k < 4; ++k)
-        ckn[f][k] = (kA == n_chunks && n_chunks >= 2) ? A.ckpt[ckpt_index<NF>(n_chunks - 1, f, k, A.n_lines, line)] : 0.0;
-  }
-  const int nB = n_chunks - k_lo;   // chunks n_chunks-1 .. k_lo
-#pragma unroll
-  for (int s = 0; s < STAGES - 1; ++s) {
-    const int kc = n_chunks - 1 - s;
-    if (s < nB) issue(stages[s], kc, kc < kA ? 0 : 3, kc < kA);
-    else cp_async_commit();
-  }
-  for (int q = 0; q < nB; ++q) {
-    const int k = n_chunks - 1 - q;
-    const int qn = q + STAGES - 1;
-    if (qn < nB) {
-      const int kc = n_chunks - 1 - qn;
-      issue(stages[qn % STAGES], kc, kc < kA ? 0 : 3, kc < kA);
-    } else {
-      cp_async_commit();
-    }
-    cp_async_wait<STAGES - 1>();
-    __syncwarp();
-    const Stage& S = stages[q % STAGES];
-    const int i0 = k * L;
-    const int len = min(L, n - i0);
-    if (k >= kA) {   // above the output range: only the anticausal state moves
-      auto srca = [&](int j, double (&v)[NF]) { stage_sample<NF, INMODE, L, !YBS>(S, 3 + j, t, v); };
-      if (chunk_is_interior<L>(i0, len, n)) anti_chunk<NF, L, FMA, false>(C, srca, i0, len, n, as);
-      else anti_chunk<NF, L, FMA, true>(C, srca, i0, len, n, as);
-      if (YBS && k - 1 >= 1 && k - 1 < kA) {
-#pragma unroll
-        for (int f = 0; f < NF; ++f)
-#pragma unroll
-          for (int kk = 0; kk < 4; ++kk) ckn[f][kk] = IFE_CACHE_HINTS ? __ldcs(A.ckpt + ckpt_index<NF>(k - 1, f, kk, A.n_lines, line)) : A.ckpt[ckpt_index<NF>(k - 1, f, kk, A.n_lines, line)];
-      }
-      __syncwarp();
-      continue;
-    }
-    if (k == 0) {
-      double v[NF];
-      stage_sample<NF, INMODE, L, !YBS>(S, 3, t, v);
-#pragma unroll
-      for (int f = 0; f < NF; ++f) rec_fill(cs[f], v[f]);
-    } else {
-      double v1[NF], v2[NF], v3[NF];
-      stage_sample<NF, INMODE, L, !YBS>(S, 2, t, v1);
-      stage_sample<NF, INMODE, L, !YBS>(S, 1, t, v2);
-      stage_sample<NF, INMODE, L, !YBS>(S, 0, t, v3);
-#pragma unroll
-      for (int f = 0; f < NF; ++f) {
-        if (YBS) {
-          cs[f].h0 = ckn[f][0]; cs[f].h1 = ckn[f][1]; cs[f].h2 = ckn[f][2]; cs[f].h3 = ckn[f][3];
-        } else {
-          cs[f].h0 = S.ck[f * 4 + 0][t];
-          cs[f].h1 = S.ck[f * 4 + 1][t];
-          cs[f].h2 = S.ck[f * 4 + 2][t];
-          cs[f].h3 = S.ck[f * 4 + 3][t];
-        }
-        cs[f].x0 = v1[f];
-        cs[f].x1 = v2[f];
-        cs[f].x2 = v3[f];
-        cs[f].x3 = 0.0;
-      }
-    }
-    if (YBS && k >= 2) {   // prefetch the next chunk's checkpoint; consumed one iteration later
-#pragma unroll
-      for (int f = 0; f < NF; ++f)
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk) ckn[f][kk] = IFE_CACHE_HINTS ? __ldcs(A.ckpt + ckpt_index<NF>(k - 1, f, kk, A.n_lines, line)) : A.ckpt[ckpt_index<NF>(k - 1, f, kk, A.n_lines, line)];
-    }
-    const size_t obase = base + (size_t)i0 * st;
-    auto src = [&](int j, double (&v)[NF]) { stage_sample<NF, INMODE, L, !YBS>(S, 3 + j, t, v); };
-    auto sink = [&](int j, const float (&o)[NF]) {
-      const size_t idx = obase + (size_t)j * st;
-      if (DIVIDE) {
-        float qv = itk_divide(o[0], o[NF - 1]);
-        if (active) {
-          if (MASKMODE == 1) qv = __ldg(A.mask_u8 + idx) != 0 ? qv : 0.0f;
-          if (MASKMODE == 2) qv = __ldg(A.mask_f32 + idx) != 0.0f ? qv : 0.0f;
-          if (IFE_CACHE_HINTS) __stcs(A.out0 + idx, qv); else A.out0[idx] = qv;
-        }
-      } else if (active) {
-        if (IFE_CACHE_HINTS) { __stcs(A.out0 + idx, o[0]); if (NF == 2) __stcs(A.out1 + idx, o[NF - 1]); }
-        else { A.out0[idx] = o[0]; if (NF == 2) A.out1[idx] = o[NF - 1]; }
-      }
-    };
-    if (YBS) {
-      // samples and replay buffer are both in shared memory: the loops need no register arrays
-      // and can stay partially rolled (smaller code, fewer instruction-cache misses)
-      if (chunk_is_interior<L>(i0, len, n)) backward_chunk<NF, L, FMA, false, kYbsUnroll>(C, src, sink, i0, len, n, cs, as, ybs);
-      else if (IFE_EDGE_HOT && len == L && i0 == 0 && n >= 2 * L) backward_chunk<NF, L, FMA, false, kYbsUnroll, 1>(C, src, sink, i0, len, n, cs, as, ybs);
-      else if (IFE_EDGE_HOT && len == L && i0 + L == n && i0 >= L) backward_chunk<NF, L, FMA, false, kYbsUnroll, 2>(C, src, sink, i0, len, n, cs, as, ybs);
-      else backward_chunk<NF, L, FMA, true, kGenUnroll>(C, src, sink, i0, len, n, cs, as, ybs);
-    } else {
-      if (chunk_is_interior<L>(i0, len, n)) backward_chunk<NF, L, FMA, false>(C, src, sink, i0, len, n, cs, as);
-      else backward_chunk<NF, L, FMA, true>(C, src, sink, i0, len, n, cs, as);
-    }
-    __syncwarp();
-  }
-  cp_async_wait<0>();
 }
 
 // ---------------------------------------------------------------------------------------
@@ -999,213 +591,6 @@ gauss_pass_x(const __grid_constant__ GaussCoef C, const __grid_constant__ PassAr
     }
     xtile_store<NF, L>(A, T, line0, i0, len, lane, xs);
   }
-}
-
-// ---------------------------------------------------------------------------------------
-// x pass, software-pipelined.  A warp owns 32 adjacent lines.  Chunk k of those lines is a
-// [32 lines] x [16 floats] tile (64 contiguous bytes per line); it is brought in by 4
-// cp.async.cg instructions per field in which four lanes cover one line's 64 bytes
-// (coalesced, every sector fully used), STAGES-1 chunks ahead.  In shared memory the four
-// 16-byte pieces of a line are XOR-swizzled with (line >> 1) & 3, which makes BOTH access
-// patterns conflict-free: the cooperative side (4 lanes per line) and the per-line side
-// (lane = line reads its 64 bytes with four LDS.128).  Results leave the same way in
-// reverse through a per-warp output tile.  Only __syncwarp is ever needed.
-// Host-checked: nx % 4 == 0, 16-byte aligned pointers.
-// ---------------------------------------------------------------------------------------
-template <int NF, int L>
-struct XStage {
-  float tile[NF][32][L];        // swizzled in 16-byte pieces
-  float hist[NF][32][4];        // samples i0-4 .. i0-1 of every line (phase B)
-  double ck[NF * 4][32];
-};
-template <int NF, int L>
-struct XOut {
-  float tile[NF][32][L];
-};
-
-__device__ __forceinline__ int xswz(int line, int piece) { return piece ^ ((line >> 1) & 3); }
-
-template <int NF, int L>
-__device__ __forceinline__ void xstage_issue(const PassArgs& A, XStage<NF, L>& S, int lane,
-                                             long long line0, int kc, bool with_hist_ckpt) {
-  static_assert(L == 16, "one chunk = four 16-byte pieces per line");
-  const int i0 = kc * L;
-  const int piece = lane & 3;
-  const bool col_ok = i0 + 4 * piece < A.n;
-#pragma unroll
-  for (int m = 0; m < 4; ++m) {
-    const int ll = (lane >> 2) + 8 * m;
-    const long long gl = line0 + ll;
-    if (gl < A.n_lines && col_ok) {
-      const size_t idx = (size_t)gl * (size_t)A.n + (size_t)(i0 + 4 * piece);
-      cp_async16(&S.tile[0][ll][4 * xswz(ll, piece)], A.in0 + idx);
-      if (NF == 2) cp_async16(&S.tile[NF - 1][ll][4 * xswz(ll, piece)], reinterpret_cast<const float*>(A.in1) + idx);
-    }
-  }
-  if (with_hist_ckpt && kc >= 1) {
-    const long long gl = line0 + lane;
-    if (gl < A.n_lines) {
-      const size_t idx = (size_t)gl * (size_t)A.n + (size_t)(i0 - 4);
-      cp_async16(&S.hist[0][lane][0], A.in0 + idx);
-      if (NF == 2) cp_async16(&S.hist[NF - 1][lane][0], reinterpret_cast<const float*>(A.in1) + idx);
-      const double* src = A.ckpt + ckpt_index<NF>(kc, 0, 0, A.n_lines, (size_t)gl);
-#pragma unroll
-      for (int k = 0; k < NF * 4; ++k) cp_async8(&S.ck[k][lane], src + (size_t)k * (size_t)A.n_lines);
-    }
-  }
-  cp_async_commit();
-}
-
-template <int NF, int L>
-__device__ __forceinline__ void xstage_read(const XStage<NF, L>& S, int lane, float (&xs)[NF][L]) {
-#pragma unroll
-  for (int f = 0; f < NF; ++f)
-#pragma unroll
-    for (int p = 0; p < 4; ++p) {
-      const float4 v = *reinterpret_cast<const float4*>(&S.tile[f][lane][4 * xswz(lane, p)]);
-      xs[f][4 * p + 0] = v.x; xs[f][4 * p + 1] = v.y; xs[f][4 * p + 2] = v.z; xs[f][4 * p + 3] = v.w;
-    }
-}
-
-#ifndef IFE_X_MINB
-#define IFE_X_MINB 1     // experiment hook: resident CTAs the x pass's registers are cut for
-#endif
-template <int NF, int L, bool FMA, int WARPS, int STAGES>
-__global__ void __launch_bounds__(WARPS * 32, IFE_X_MINB)
-gauss_pass_x_async(const __grid_constant__ GaussCoef C, const __grid_constant__ PassArgs A) {
-  extern __shared__ __align__(16) unsigned char xasync_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  XStage<NF, L>* stages = reinterpret_cast<XStage<NF, L>*>(xasync_smem) + warp * STAGES;
-  XOut<NF, L>& O = reinterpret_cast<XOut<NF, L>*>(reinterpret_cast<XStage<NF, L>*>(xasync_smem) + WARPS * STAGES)[warp];
-  const long long line0 = ((long long)blockIdx.x * WARPS + warp) * 32;
-  if (line0 >= A.n_lines) return;   // whole warp exits together
-  const long long line = line0 + lane;
-  const bool active = line < A.n_lines;
-  const int n = A.n;
-  const int n_chunks = (n + L - 1) / L;
-
-  float xs[NF][L];
-  Rec cs[NF];
-  Rec as[NF];
-
-  // ---- phase A ----
-#pragma unroll
-  for (int s = 0; s < STAGES - 1; ++s) {
-    if (s < n_chunks) xstage_issue<NF, L>(A, stages[s], lane, line0, s, false);
-    else cp_async_commit();
-  }
-  for (int k = 0; k < n_chunks; ++k) {
-    const int kn = k + STAGES - 1;
-    if (kn < n_chunks) xstage_issue<NF, L>(A, stages[kn % STAGES], lane, line0, kn, false);
-    else cp_async_commit();
-    cp_async_wait<STAGES - 1>();
-    __syncwarp();
-    xstage_read<NF, L>(stages[k % STAGES], lane, xs);
-    __syncwarp();
-    const int i0 = k * L;
-    const int len = min(L, n - i0);
-    if (k == 0) {
-#pragma unroll
-      for (int f = 0; f < NF; ++f) rec_fill(cs[f], (double)xs[f][0]);
-    } else if (active) {
-#pragma unroll
-      for (int f = 0; f < NF; ++f) {
-        A.ckpt[ckpt_index<NF>(k, f, 0, A.n_lines, line)] = cs[f].h0;
-        A.ckpt[ckpt_index<NF>(k, f, 1, A.n_lines, line)] = cs[f].h1;
-        A.ckpt[ckpt_index<NF>(k, f, 2, A.n_lines, line)] = cs[f].h2;
-        A.ckpt[ckpt_index<NF>(k, f, 3, A.n_lines, line)] = cs[f].h3;
-      }
-    }
-    {
-      const RegSrc<NF, L> src{xs};
-      if (len == L && i0 >= 4) forward_chunk<NF, L, FMA, false>(C, src, i0, len, cs);
-      else forward_chunk<NF, L, FMA, true>(C, src, i0, len, cs);
-    }
-    if (k == n_chunks - 1) {
-      float vlast[NF];
-#pragma unroll
-      for (int f = 0; f < NF; ++f) vlast[f] = xs[f][0];
-#pragma unroll
-      for (int j = 1; j < L; ++j)
-        if (j < len) {
-#pragma unroll
-          for (int f = 0; f < NF; ++f) vlast[f] = xs[f][j];
-        }
-#pragma unroll
-      for (int f = 0; f < NF; ++f) rec_fill(as[f], (double)vlast[f]);
-    }
-  }
-  cp_async_wait<0>();
-  __threadfence_block();
-
-  // ---- phase B ----
-#pragma unroll
-  for (int s = 0; s < STAGES - 1; ++s) {
-    const int kc = n_chunks - 1 - s;
-    if (kc >= 0) xstage_issue<NF, L>(A, stages[s], lane, line0, kc, true);
-    else cp_async_commit();
-  }
-  for (int q = 0; q < n_chunks; ++q) {
-    const int k = n_chunks - 1 - q;
-    const int qn = q + STAGES - 1;
-    if (qn < n_chunks) xstage_issue<NF, L>(A, stages[qn % STAGES], lane, line0, n_chunks - 1 - qn, true);
-    else cp_async_commit();
-    cp_async_wait<STAGES - 1>();
-    __syncwarp();
-    const XStage<NF, L>& S = stages[q % STAGES];
-    xstage_read<NF, L>(S, lane, xs);
-    const int i0 = k * L;
-    const int len = min(L, n - i0);
-    if (k == 0) {
-#pragma unroll
-      for (int f = 0; f < NF; ++f) rec_fill(cs[f], (double)xs[f][0]);
-    } else {
-#pragma unroll
-      for (int f = 0; f < NF; ++f) {
-        const float4 h = *reinterpret_cast<const float4*>(&S.hist[f][lane][0]);
-        cs[f].h0 = S.ck[f * 4 + 0][lane];
-        cs[f].h1 = S.ck[f * 4 + 1][lane];
-        cs[f].h2 = S.ck[f * 4 + 2][lane];
-        cs[f].h3 = S.ck[f * 4 + 3][lane];
-        cs[f].x0 = (double)h.w;
-        cs[f].x1 = (double)h.z;
-        cs[f].x2 = (double)h.y;
-        cs[f].x3 = 0.0;
-      }
-    }
-    __syncwarp();   // stage fully consumed by every lane before any lane refills it
-    {
-      const RegSrc<NF, L> src{xs};
-      const RegSink<NF, L> sink{xs};
-      if (chunk_is_interior<L>(i0, len, n)) backward_chunk<NF, L, FMA, false>(C, src, sink, i0, len, n, cs, as);
-      else backward_chunk<NF, L, FMA, true>(C, src, sink, i0, len, n, cs, as);
-    }
-    // results -> swizzled output tile -> coalesced 16-byte stores
-#pragma unroll
-    for (int f = 0; f < NF; ++f)
-#pragma unroll
-      for (int p = 0; p < 4; ++p)
-        *reinterpret_cast<float4*>(&O.tile[f][lane][4 * xswz(lane, p)]) =
-            make_float4(xs[f][4 * p], xs[f][4 * p + 1], xs[f][4 * p + 2], xs[f][4 * p + 3]);
-    __syncwarp();
-    {
-      const int piece = lane & 3;
-      const bool col_ok = i0 + 4 * piece < n;
-#pragma unroll
-      for (int m = 0; m < 4; ++m) {
-        const int ll = (lane >> 2) + 8 * m;
-        const long long gl = line0 + ll;
-        if (gl < A.n_lines && col_ok) {
-          const size_t idx = (size_t)gl * (size_t)n + (size_t)(i0 + 4 * piece);
-          *reinterpret_cast<float4*>(A.out0 + idx) = *reinterpret_cast<const float4*>(&O.tile[0][ll][4 * xswz(ll, piece)]);
-          if (NF == 2)
-            *reinterpret_cast<float4*>(A.out1 + idx) = *reinterpret_cast<const float4*>(&O.tile[NF - 1][ll][4 * xswz(ll, piece)]);
-        }
-      }
-    }
-    __syncwarp();
-  }
-  cp_async_wait<0>();
 }
 
 }  // namespace ife

@@ -104,10 +104,7 @@ uint64_t ife_cuda_launch_count(const ife_cuda_ctx* ctx);
  * For benchmarks that report bytes moved per kernel. */
 int ife_cuda_last_work_dims(const ife_cuda_ctx* ctx, int dims[3]);
 
-/* Tuning / debugging switches.  "async_passes" (default 1): use the cp.async software-
- * pipelined Gaussian pass kernels; 0 selects the plain register-staged kernels (same
- * results bit for bit; kept as the fallback for layouts the pipelined kernels reject).
- * "support_box" (default 1): the calls whose every result is masked
+/* Tuning / debugging switches.  "support_box" (default 1): the calls whose every result is masked
  * (ife_cuda_emphysema_features / _histograms / _histograms_batch) smooth only what an in-mask
  * voxel can see -- the mask's bounding box grown by the one-voxel stencil reach, smoothed as a
  * dense cropped copy (outside the mask both fields of the normalized convolution are exact
@@ -122,7 +119,8 @@ int ife_cuda_last_work_dims(const ife_cuda_ctx* ctx, int dims[3]);
  * "tma_passes" (default 1): normalized convolution with a uint8 certainty on volumes with
  * nx % 16 == 0, or with a float certainty and nx % 4 == 0 (with or without output mask), and the plain
  * Gaussian with nx % 4 == 0 run the tensor-map staged, field-per-warp pass kernels
- * (csrc/iir_tma.cuh); 0 selects the cp.async kernels (same results bit for bit).
+ * (csrc/iir_tma.cuh); 0 selects the plain register-staged kernels, which every other layout
+ * runs (same results bit for bit).
  * "march4" (default 1): the fused feature kernel owns four x-adjacent voxels per thread when
  * nx % 4 == 0 and the pointers are 16-byte aligned (csrc/features_march4.cuh); 0 selects the
  * one-voxel-per-thread kernel (same results bit for bit).

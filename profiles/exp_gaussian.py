@@ -35,6 +35,6 @@ for tma in (1, 0):
     cur = out.clone()
     same = None if ref is None else bool(torch.equal(cur, ref))
     ref = cur
-    print("gaussian sigma", sigma, "tma" if tma else "cp.async", t, "sum_passes",
+    print("gaussian sigma", sigma, "tma" if tma else "plain", t, "sum_passes",
           round(sum(v for k, v in t.items() if "pass" in k), 4), "identical to previous:", same, flush=True)
 ctx.close()

@@ -39,6 +39,6 @@ for mask_kind in ("ones", "lung"):
         cur = out[0, 0].clone()
         same = None if ref is None else bool(torch.equal(cur, ref))
         ref = cur
-        print(os.path.basename(os.environ.get("IFE_CUDA_LIB", "product")), mask_kind, "tma" if tma else "cp.async", t,
+        print(os.path.basename(os.environ.get("IFE_CUDA_LIB", "product")), mask_kind, "tma" if tma else "plain", t,
               "sum_passes", round(sum(v for k, v in t.items() if "pass" in k), 4), "blur identical to previous:", same, flush=True)
 ctx.close()

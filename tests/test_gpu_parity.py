@@ -128,7 +128,7 @@ def test_normalized_gaussian_bit_exact(ctx, oracle, arith):
 @pytest.mark.parametrize("arith", [0, 1])
 def test_tensor_map_passes_bit_exact(ctx, oracle, arith):
     """The tensor-map staged, field-per-warp passes (csrc/iir_tma.cuh; taken when nx % 16 == 0
-    with a uint8 certainty) against the cp.async passes and the oracle: whole tiles, ragged
+    with a uint8 certainty) against the plain register-staged passes and the oracle: whole tiles, ragged
     tiles in every direction (nx, ny not multiples of 32, lines that are not whole chunks),
     lines shorter than one chunk, the smallest volume ITK accepts."""
     shapes = [((40, 64, 96), 1.2), ((37, 45, 48), 2.4), ((4, 4, 16), 0.6), ((5, 6, 32), 1.0),
@@ -147,7 +147,7 @@ def test_tensor_map_passes_bit_exact(ctx, oracle, arith):
             finally:
                 ctx.set_option("tma_passes", 1)
             n, worst = mismatch_report(got, old)
-            assert n == 0, "%s sigma=%g: %d values differ from the cp.async passes (max %g)" % (shape, sigma, n, worst)
+            assert n == 0, "%s sigma=%g: %d values differ from the plain passes (max %g)" % (shape, sigma, n, worst)
             if np.prod(shape) < 200_000:
                 ref = oracle.normalized_gaussian(img, m8.astype(np.float32), sigma, arith=arith)
                 assert mismatch_report(got, ref)[0] == 0, "%s sigma=%g vs oracle" % (shape, sigma)
@@ -179,7 +179,7 @@ def test_tensor_map_plain_gaussian_bit_exact(ctx, oracle, arith):
             finally:
                 ctx.set_option("tma_passes", 1)
             n, worst = mismatch_report(got, old)
-            assert n == 0, "%s sigma=%g: %d values differ from the cp.async passes (max %g)" % (shape, sigma, n, worst)
+            assert n == 0, "%s sigma=%g: %d values differ from the plain passes (max %g)" % (shape, sigma, n, worst)
             if np.prod(shape) < 200_000:
                 ref = oracle.smoothing_recursive_gaussian(img, sigma, arith=arith)
                 assert mismatch_report(got, ref)[0] == 0, "%s sigma=%g vs oracle" % (shape, sigma)
@@ -212,12 +212,12 @@ def test_tensor_map_float_certainty_bit_exact(ctx, oracle, arith):
             finally:
                 ctx.set_option("tma_passes", 1)
             n, worst = mismatch_report(got, old)
-            assert n == 0, "%s sigma=%g: %d values differ from the cp.async passes (max %g)" % (shape, sigma, n, worst)
+            assert n == 0, "%s sigma=%g: %d values differ from the plain passes (max %g)" % (shape, sigma, n, worst)
             if np.prod(shape) < 200_000:
                 ref = oracle.normalized_gaussian(img, cert, sigma, arith=arith)
                 assert mismatch_report(got, ref)[0] == 0, "%s sigma=%g vs oracle" % (shape, sigma)
         # the output mask (the tool's -m flag) is applied where the y pass divides: same answer as masking
-        # afterwards and as the cp.async kernels, float and uint8 certainty, ragged tiles
+        # afterwards and as the plain kernels, float and uint8 certainty, ragged tiles
         for shape in ((24, 40, 64), (21, 37, 48), (9, 50, 16)):
             img = synth.ct_like(shape, seed=9, n_blobs=5)
             for cert in ((np.random.default_rng(6).uniform(0, 1, shape) < 0.6).astype(np.float32),
@@ -370,12 +370,13 @@ def test_emphysema_features_anisotropic_spacing(ctx, oracle):
         assert np.abs(got.astype(np.int64) - ref_counts.astype(np.int64)).sum() <= 2
 
 
-def test_support_box_is_invisible(ctx, oracle):
+def test_support_box_is_invisible_to_both_pass_families(ctx, oracle):
     """Masked paths smooth only the mask's bounding box grown by the stencil reach (lines that
     miss it are skipped, the sweeps along a line stop at it).  No result may change: the same
-    call with the option off, and the oracle, give identical outputs; an empty mask and a mask
-    touching the volume corner work too."""
-    shape = (40, 64, 96)                      # nz, ny, nx: every pass takes its pipelined kernel
+    call with the option off, the same call through the plain pass kernels instead of the
+    tensor-map ones, and the oracle give identical outputs; an empty mask and a mask touching
+    the volume corner work too."""
+    shape = (40, 64, 96)                      # nz, ny, nx: every pass takes its tensor-map kernel
     sigmas = [0.6, 2.4]
     img = synth.ct_like(shape, seed=31, n_blobs=10)
     zz, yy, xx = np.ogrid[:shape[0], :shape[1], :shape[2]]
@@ -395,11 +396,11 @@ def test_support_box_is_invisible(ctx, oracle):
         assert mismatch_report(out[s, :2], ref[:2])[0] == 0
         assert_eigen_parity(np.moveaxis(out[s, 2:], 0, -1), np.moveaxis(ref[2:], 0, -1), "box sigma=%g" % sigma)
     assert np.all(ctx.emphysema_features(img, np.zeros(shape, np.uint8), sigmas) == 0)
-    ctx.set_option("async_passes", 0)         # the plain pass kernels take the same windows
+    ctx.set_option("tma_passes", 0)           # the plain pass kernels take the same windows
     try:
         assert bits_equal(ctx.emphysema_features(img, corner, sigmas), out)
     finally:
-        ctx.set_option("async_passes", 1)
+        ctx.set_option("tma_passes", 1)
     # histograms: the box is also clipped to the ROI list's bounding box
     edges = _edges_for(oracle, img, blob, sigmas, 12)
     rois = np.array([[60, 12, 22, 9, 7, 5], [72, 20, 26, 11, 9, 6]], np.int32)   # x,y,z,sx,sy,sz
