@@ -331,7 +331,7 @@ int smooth_volume(ife_cuda_ctx* ctx, const float* in0, const void* cert, bool ce
                 nzb);
   if (!(sigma > 0.0)) return fail(ctx, IFE_E_INVALID, "sigma must be positive (got %g)", sigma);
   if (keep0 < 0 || keep1 > nzb || keep0 >= keep1) return fail(ctx, IFE_E_INVALID, "bad plane range");
-  // Support box (masked paths, compute_support_box): nothing outside it is ever read, so the z
+  // Support box (masked paths, plan_masked): nothing outside it is ever read, so the z
   // pass only keeps the box's planes (below them the causal sweep alone runs, above them the
   // anticausal one), the x pass runs the rows of those planes, and the y pass the columns
   // (x, z) that cross the box, restricted to its y range.  Columns come in whole warps of 32.
@@ -556,17 +556,6 @@ void finish_support_box(const ife_cuda_ctx* ctx, int slot, int nx, int ny, int n
   }
 }
 
-// the three steps on the context's stream; waits for the stream once
-int compute_support_box(ife_cuda_ctx* ctx, const uint8_t* d_mask, int nx, int ny, int nz,
-                        const int* rois, int n_roi, int box[6], bool* have) {
-  *have = support_box_usable(ctx, d_mask, nx, ny, nz);
-  if (!*have) return IFE_OK;
-  IFE_TRY(launch_support_box(ctx, d_mask, nx, ny, nz, ctx->stream(), 0));
-  IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  finish_support_box(ctx, 0, nx, ny, nz, rois, n_roi, box);
-  return IFE_OK;
-}
-
 // ---------------------------------------------------------------------------------------
 // Masked smoothing.  With a mask c in {0, != 0} both fields of the normalized convolution, c*T
 // and c, are EXACT zeros outside the mask's bounding box.  The recursion of a line that has
@@ -645,23 +634,44 @@ int plan_masked(ife_cuda_ctx* ctx, bool have_box, int slot, const float* d_img, 
   return IFE_OK;
 }
 
-// ROI list in crop coordinates, clipped to the crop (in-mask voxels all lie inside it)
-std::vector<int> rois_in_crop(const MaskedPlan& P, const int* rois, int n_roi) {
-  std::vector<int> r((size_t)n_roi * 6);
-  for (int i = 0; i < n_roi; ++i) {
-    int lo[3], hi[3];
-    bool empty = false;
-    for (int d = 0; d < 3; ++d) {
-      lo[d] = std::max(rois[6 * i + d] - P.org[d], 0);
-      hi[d] = std::min(rois[6 * i + d] + rois[6 * i + 3 + d] - P.org[d], P.cdim[d]);
-      empty = empty || lo[d] >= hi[d];
-    }
-    for (int d = 0; d < 3; ++d) {
-      r[6 * i + d] = empty ? 0 : lo[d];
-      r[6 * i + 3 + d] = empty ? 0 : hi[d] - lo[d];
-    }
+// The same for one scan on the context's stream: the support box's reduction, one wait for its
+// extents, then the plan.
+int plan_masked(ife_cuda_ctx* ctx, const float* d_img, const uint8_t* d_mask, int nx, int ny, int nz,
+                const int* rois, int n_roi, MaskedPlan* P) {
+  const bool have_box = support_box_usable(ctx, d_mask, nx, ny, nz);
+  if (have_box) {
+    IFE_TRY(launch_support_box(ctx, d_mask, nx, ny, nz, ctx->stream(), 0));
+    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
   }
-  return r;
+  return plan_masked(ctx, have_box, 0, d_img, d_mask, nx, ny, nz, rois, n_roi, P);
+}
+
+// Upload a scan's ROI list to d_rois on the context's stream.  With a crop the list is moved into
+// crop coordinates and clipped to the crop (in-mask voxels all lie inside it) in `moved`, which
+// must outlive the copy.
+int upload_rois(ife_cuda_ctx* ctx, const MaskedPlan& P, const int* rois, int n_roi, int* d_rois,
+                std::vector<int>* moved) {
+  if (n_roi == 0) return IFE_OK;
+  if (P.cropped) {
+    moved->assign((size_t)n_roi * 6, 0);
+    for (int i = 0; i < n_roi; ++i) {
+      int lo[3], hi[3];
+      bool empty = false;
+      for (int d = 0; d < 3; ++d) {
+        lo[d] = std::max(rois[6 * i + d] - P.org[d], 0);
+        hi[d] = std::min(rois[6 * i + d] + rois[6 * i + 3 + d] - P.org[d], P.cdim[d]);
+        empty = empty || lo[d] >= hi[d];
+      }
+      for (int d = 0; d < 3; ++d) {
+        (*moved)[6 * i + d] = empty ? 0 : lo[d];
+        (*moved)[6 * i + 3 + d] = empty ? 0 : hi[d] - lo[d];
+      }
+    }
+    rois = moved->data();
+  }
+  IFE_CUDA_TRY(ctx, cudaMemcpyAsync(d_rois, rois, (size_t)n_roi * 6 * sizeof(int), cudaMemcpyHostToDevice,
+                                    ctx->stream()));
+  return IFE_OK;
 }
 
 // blur (full layout) <- normalized Gaussian of (img, mask) at `sigma`, valid wherever P.box says
@@ -737,9 +747,6 @@ void launch_features_t(bool unit, dim3 grid, dim3 block, size_t smem, cudaStream
   else if (unit) features_kernel<BM, HIST, true, false><<<grid, block, smem, st>>>(S, A);
   else features_kernel<BM, HIST, false, false><<<grid, block, smem, st>>>(S, A);
 }
-
-// ROI lists longer than this take the packed-bin path (one block per ROI)
-constexpr int kManyRois = 192;
 
 // shared memory of the z-march kernel's histogram sink: padded edge rows + private counter columns
 inline size_t march_hist_smem(int nfeat, int n_edges) {
@@ -834,12 +841,72 @@ inline bool is_unit_spacing(const double spacing[3]) {
   return spacing[0] == 1.0 && spacing[1] == 1.0 && spacing[2] == 1.0;
 }
 
+// ROI lists longer than this take the packed-bin path (one block per ROI)
+constexpr int kManyRois = 192;
+
+// The histograms of one scan (ife_cuda_emphysema_histograms and each scan of _histograms_batch):
+// per scale the normalized convolution of the plan's volume and the fused kernel's histogram sink,
+// on the crop when there is one, since no feature volume leaves the call.  d_edges:
+// [n_sigma*8][n_edges]; d_rois: the scan's ROI list in the plan's frame (upload_rois); d_counts:
+// [max(n_roi,1)][n_sigma*8][n_edges+1], zeroed.  Of the workspace only the smoothing buffers and
+// ws.packed are touched: a batch keeps its upload and count slots in ws.in_*, ws.out[*], ws.counts.
+int bin_masked_scan(ife_cuda_ctx* ctx, const MaskedPlan& P, const float* d_img, const uint8_t* d_mask,
+                    int nx, int ny, int nz, const double spacing[3], const double* sigmas, int n_sigma,
+                    const float* d_edges, int n_edges, const int* d_rois, int n_roi, uint32_t* d_counts) {
+  if (P.have_box && P.empty) return IFE_OK;   // no voxel is wanted
+  // Many ROIs (MakeBagDense, large MakeBag runs): the per-voxel search through the ROI list of
+  // the brick kernel does not scale, so the fused kernel leaves packed bin indices and one
+  // block per ROI counts its box (roi_hist_packed_kernel).
+  const bool many_rois = n_roi > kManyRois && n_edges <= 253 && march_hist_fits(8, n_edges) &&
+                         (long long)nx * ny < (1LL << 28);
+  if (many_rois) IFE_TRY(ctx->ws.packed.reserve(ctx, (size_t)nx * ny * nz * sizeof(unsigned long long)));
+  const int fx = P.cropped ? P.cdim[0] : nx, fy = P.cropped ? P.cdim[1] : ny, fz = P.cropped ? P.cdim[2] : nz;
+  const int nb = n_edges + 1;
+  const StencilCoef S = make_stencil_coef(spacing);
+  float* blur = P.cropped ? (float*)ctx->ws.crop_blur.ptr : (float*)ctx->ws.blur.ptr;
+  for (int s = 0; s < n_sigma; ++s) {
+    IFE_TRY(smooth_masked(ctx, P, d_img, d_mask, blur, nx, ny, nz, spacing, sigmas[s], false));
+    FeatArgs A;
+    std::memset(&A, 0, sizeof(A));
+    A.vol = blur; A.mask_u8 = P.mask;
+    A.nx = fx; A.ny = fy; A.nzb = fz; A.zb0 = 0; A.zb1 = fz;
+    A.hist.edges = d_edges + (size_t)s * 8 * n_edges;
+    A.hist.counts = d_counts + (size_t)s * 8 * nb;
+    A.hist.n_edges = n_edges;
+    A.hist.stride_roi = (long long)n_sigma * 8 * nb;
+    if (many_rois) {
+      A.hist.packed = (unsigned long long*)ctx->ws.packed.ptr;
+      IFE_TRY(launch_features(ctx, 0, S, A, is_unit_spacing(spacing)));
+      ProfScope prof(ctx, K_OTHER);
+      roi_hist_packed_kernel<<<(unsigned)n_roi, 256, (size_t)8 * nb * sizeof(uint32_t), ctx->stream()>>>(
+          A.hist.packed, fx, fy, d_rois, nb, A.hist.counts, A.hist.stride_roi);
+      ctx->launches++;
+      IFE_CUDA_TRY(ctx, cudaGetLastError());
+    } else {
+      A.hist.rois = d_rois; A.hist.n_roi = n_roi;
+      IFE_TRY(launch_features(ctx, 0, S, A, is_unit_spacing(spacing)));
+    }
+  }
+  return IFE_OK;
+}
+
 int check_dims(ife_cuda_ctx* ctx, const int dims[3], const double spacing[3]) {
   if (!dims || !spacing) return fail(ctx, IFE_E_INVALID, "dims/spacing must not be null");
   for (int d = 0; d < 3; ++d) {
     if (dims[d] <= 0) return fail(ctx, IFE_E_INVALID, "dims[%d] = %d must be positive", d, dims[d]);
     if (!(spacing[d] > 0.0))
       return fail(ctx, IFE_E_INVALID, "spacing[%d] = %g must be positive", d, spacing[d]);
+  }
+  return IFE_OK;
+}
+
+// Every box of an ROI list (host, n_roi x {x0,y0,z0,sx,sy,sz}) is non-empty and inside the image.
+int check_rois(ife_cuda_ctx* ctx, const int* rois, int n_roi, const int dims[3]) {
+  for (int r = 0; r < n_roi; ++r) {
+    const int* b = rois + 6 * r;
+    if (b[0] < 0 || b[1] < 0 || b[2] < 0 || b[3] <= 0 || b[4] <= 0 || b[5] <= 0 ||
+        b[0] + b[3] > dims[0] || b[1] + b[4] > dims[1] || b[2] + b[5] > dims[2])
+      return fail(ctx, IFE_E_INVALID, "ROI %d is not inside the image", r);
   }
   return IFE_OK;
 }
@@ -854,6 +921,26 @@ int stage_in(ife_cuda_ctx* ctx, DeviceBuffer& buf, const T* src, size_t count, i
   IFE_CUDA_TRY(ctx, cudaMemcpyAsync(buf.ptr, src, count * sizeof(T), cudaMemcpyHostToDevice,
                                     ctx->stream()));
   *dev = (const T*)buf.ptr;
+  return IFE_OK;
+}
+
+// Where the kernels write an output of `count` elements: with IFE_MEM_HOST the workspace buffer
+// `buf`, which finish_out copies to the caller's `dst`; else `dst` itself.
+template <typename T>
+int stage_out(ife_cuda_ctx* ctx, DeviceBuffer& buf, T* dst, size_t count, int mem, T** dev) {
+  *dev = dst;
+  if (mem != IFE_MEM_HOST) return IFE_OK;
+  IFE_TRY(buf.reserve(ctx, count * sizeof(T)));
+  *dev = (T*)buf.ptr;
+  return IFE_OK;
+}
+
+// With IFE_MEM_HOST: copy a staged output back on the context's stream and wait for it.
+template <typename T>
+int finish_out(ife_cuda_ctx* ctx, T* dst, const T* dev, size_t count, int mem) {
+  if (mem != IFE_MEM_HOST) return IFE_OK;
+  IFE_CUDA_TRY(ctx, cudaMemcpyAsync(dst, dev, count * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream()));
+  IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
   return IFE_OK;
 }
 
@@ -1123,19 +1210,11 @@ int ife_cuda_gaussian(ife_cuda_ctx* ctx, const float* in, float* out, const int 
   IFE_TRY(reserve_smoothing(ctx, 1, dims[0], dims[1], dims[2]));
   const float* d_in;
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, in, n, mem, &d_in));
-  float* d_out = out;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, n * sizeof(float)));
-    d_out = (float*)ctx->ws.out[0].ptr;
-  }
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out, n, mem, &d_out));
   IFE_TRY(smooth_volume(ctx, d_in, nullptr, false, d_out, dims[0], dims[1], dims[2], 0, dims[2], spacing,
                         sigma, nullptr, nullptr));
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, n * sizeof(float), cudaMemcpyDeviceToHost,
-                                      ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, out, d_out, n, mem);
 }
 
 int ife_cuda_normalized_gaussian(ife_cuda_ctx* ctx, const float* image, const float* cert_f32,
@@ -1155,21 +1234,13 @@ int ife_cuda_normalized_gaussian(ife_cuda_ctx* ctx, const float* image, const fl
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, image, n, mem, &d_img));
   if (cert_f32) IFE_TRY(stage_in(ctx, ctx->ws.in_mask, cert_f32, n, mem, &d_cf));
   else IFE_TRY(stage_in(ctx, ctx->ws.in_mask, cert_u8, n, mem, &d_cu));
-  float* d_out = out;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, n * sizeof(float)));
-    d_out = (float*)ctx->ws.out[0].ptr;
-  }
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out, n, mem, &d_out));
   const void* cert = cert_f32 ? (const void*)d_cf : (const void*)d_cu;
   IFE_TRY(smooth_volume(ctx, d_img, cert, cert_u8 != nullptr, d_out, dims[0], dims[1], dims[2],
                         0, dims[2], spacing, sigma, mask_output ? d_cu : nullptr,
                         mask_output ? d_cf : nullptr));
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, n * sizeof(float), cudaMemcpyDeviceToHost,
-                                      ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, out, d_out, n, mem);
 }
 
 int ife_cuda_gradient_magnitude(ife_cuda_ctx* ctx, const float* in, const float* mask_f32,
@@ -1186,22 +1257,14 @@ int ife_cuda_gradient_magnitude(ife_cuda_ctx* ctx, const float* in, const float*
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, in, n, mem, &d_in));
   if (mask_f32) IFE_TRY(stage_in(ctx, ctx->ws.in_mask, mask_f32, n, mem, &d_mf));
   else if (mask_u8) IFE_TRY(stage_in(ctx, ctx->ws.in_mask, mask_u8, n, mem, &d_mu));
-  float* d_out = out;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, n * sizeof(float)));
-    d_out = (float*)ctx->ws.out[0].ptr;
-  }
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out, n, mem, &d_out));
   FeatArgs A;
   std::memset(&A, 0, sizeof(A));
   A.vol = d_in; A.mask_u8 = d_mu; A.mask_f32 = d_mf; A.out[0] = d_out;
   A.nx = dims[0]; A.ny = dims[1]; A.nzb = dims[2]; A.zb0 = 0; A.zb1 = dims[2];
   IFE_TRY(launch_features(ctx, 2, make_stencil_coef(spacing), A, is_unit_spacing(spacing)));
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, n * sizeof(float), cudaMemcpyDeviceToHost,
-                                      ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, out, d_out, n, mem);
 }
 
 int ife_cuda_hessian_eigen_features(ife_cuda_ctx* ctx, const float* image, const uint8_t* mask,
@@ -1224,11 +1287,8 @@ int ife_cuda_hessian_eigen_features(ife_cuda_ctx* ctx, const float* image, const
                           dims[2], 0, dims[2], spacing, sigma, nullptr, nullptr));
     src = (const float*)ctx->ws.blur.ptr;
   }
-  float* d_out = out6;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, 6 * n * sizeof(float)));
-    d_out = (float*)ctx->ws.out[0].ptr;
-  }
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out6, 6 * n, mem, &d_out));
   FeatArgs A;
   std::memset(&A, 0, sizeof(A));
   A.vol = src; A.mask_u8 = d_mask;
@@ -1236,12 +1296,7 @@ int ife_cuda_hessian_eigen_features(ife_cuda_ctx* ctx, const float* image, const
   A.nx = dims[0]; A.ny = dims[1]; A.nzb = dims[2]; A.zb0 = 0; A.zb1 = dims[2];
   A.dy_bug = (flags & IFE_FDHF_TOOL_DY_BUG) ? 1 : 0;
   IFE_TRY(launch_features(ctx, 1, make_stencil_coef(spacing), A, is_unit_spacing(spacing)));
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out6, d_out, 6 * n * sizeof(float), cudaMemcpyDeviceToHost,
-                                      ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, out6, d_out, 6 * n, mem);
 }
 
 int ife_cuda_hessian(ife_cuda_ctx* ctx, const float* image, float* out6, const int dims[3],
@@ -1253,23 +1308,15 @@ int ife_cuda_hessian(ife_cuda_ctx* ctx, const float* image, float* out6, const i
   const size_t n = (size_t)dims[0] * dims[1] * dims[2];
   const float* d_img;
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, image, n, mem, &d_img));
-  float* d_out = out6;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, 6 * n * sizeof(float)));
-    d_out = (float*)ctx->ws.out[0].ptr;
-  }
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out6, 6 * n, mem, &d_out));
   FeatArgs A;
   std::memset(&A, 0, sizeof(A));
   A.vol = d_img;
   for (int k = 0; k < 6; ++k) A.out[k] = d_out + (size_t)k * n;
   A.nx = dims[0]; A.ny = dims[1]; A.nzb = dims[2]; A.zb0 = 0; A.zb1 = dims[2];
   IFE_TRY(launch_features(ctx, 3, make_stencil_coef(spacing), A, is_unit_spacing(spacing)));
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out6, d_out, 6 * n * sizeof(float), cudaMemcpyDeviceToHost,
-                                      ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, out6, d_out, 6 * n, mem);
 }
 
 int ife_cuda_emphysema_features(ife_cuda_ctx* ctx, const float* image, const uint8_t* mask,
@@ -1294,11 +1341,8 @@ int ife_cuda_emphysema_features(ife_cuda_ctx* ctx, const float* image, const uin
     if (n_sigma > 1) IFE_TRY(ctx->ws.out[1].reserve(ctx, 8 * n * sizeof(float)));
   }
   const StencilCoef S = make_stencil_coef(spacing);
-  int box[6];         // all eight outputs are masked: smooth only what in-mask voxels can see
-  bool have_box;
-  IFE_TRY(compute_support_box(ctx, d_mask, nx, ny, nz, nullptr, 0, box, &have_box));
-  MaskedPlan plan;
-  IFE_TRY(plan_masked(ctx, have_box, 0, d_img, d_mask, nx, ny, nz, nullptr, 0, &plan));
+  MaskedPlan plan;    // all eight outputs are masked: smooth only what in-mask voxels can see
+  IFE_TRY(plan_masked(ctx, d_img, d_mask, nx, ny, nz, nullptr, 0, &plan));
   // Option "overlap_scales" (device-resident calls with several scales): the Gaussian passes run
   // on the context's high-priority stream one scale ahead of the fused feature kernel, which
   // stays on the main stream and fills the issue slots the FP64-latency-bound passes leave
@@ -1360,12 +1404,7 @@ int ife_cuda_emphysema_histograms(ife_cuda_ctx* ctx, const float* image, const u
   IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int nx = dims[0], ny = dims[1], nz = dims[2];
   const size_t n = (size_t)nx * ny * nz;
-  for (int r = 0; r < n_roi; ++r) {
-    const int* b = rois + 6 * r;
-    if (b[0] < 0 || b[1] < 0 || b[2] < 0 || b[3] <= 0 || b[4] <= 0 || b[5] <= 0 ||
-        b[0] + b[3] > nx || b[1] + b[4] > ny || b[2] + b[5] > nz)
-      return fail(ctx, IFE_E_INVALID, "ROI %d is not inside the image", r);
-  }
+  IFE_TRY(check_rois(ctx, rois, n_roi, dims));
   IFE_TRY(reserve_smoothing(ctx, 2, nx, ny, nz));
   IFE_TRY(ctx->ws.blur.reserve(ctx, n * sizeof(float)));
   const float* d_img;
@@ -1373,76 +1412,30 @@ int ife_cuda_emphysema_histograms(ife_cuda_ctx* ctx, const float* image, const u
   IFE_TRY(stage_image(ctx, image, n, mem, &d_img));
   IFE_TRY(stage_in(ctx, ctx->ws.in_mask, mask, n, mem, &d_mask));
 
-  const int rows = n_sigma * 8, nb = n_edges + 1, R = std::max(n_roi, 1);
-  const size_t n_counts = (size_t)R * rows * nb;
+  const int rows = n_sigma * 8, R = std::max(n_roi, 1);
+  const size_t n_counts = (size_t)R * rows * (n_edges + 1);
   // parameter arrays are host pointers; counts follows `mem`
   IFE_TRY(ctx->ws.edges.reserve(ctx, (size_t)rows * n_edges * sizeof(float)));
   IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws.edges.ptr, edges, (size_t)rows * n_edges * sizeof(float),
                                     cudaMemcpyHostToDevice, ctx->stream()));
-  const int* d_rois = nullptr;
+  int* d_rois = nullptr;
   if (n_roi > 0) {   // uploaded below, once the crop frame is known
     IFE_TRY(ctx->ws.rois.reserve(ctx, (size_t)n_roi * 6 * sizeof(int)));
-    d_rois = (const int*)ctx->ws.rois.ptr;
+    d_rois = (int*)ctx->ws.rois.ptr;
   }
-  uint32_t* d_counts = counts;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.counts.reserve(ctx, n_counts * sizeof(uint32_t)));
-    d_counts = (uint32_t*)ctx->ws.counts.ptr;
-  }
+  uint32_t* d_counts;
+  IFE_TRY(stage_out(ctx, ctx->ws.counts, counts, n_counts, mem, &d_counts));
   IFE_CUDA_TRY(ctx, cudaMemsetAsync(d_counts, 0, n_counts * sizeof(uint32_t), ctx->stream()));
-
-  // Many ROIs (MakeBagDense, large MakeBag runs): the per-voxel search through the ROI list of
-  // the brick kernel does not scale, so the fused kernel leaves packed bin indices and one
-  // block per ROI counts its box (roi_hist_packed_kernel).
-  const bool many_rois = n_roi > kManyRois && n_edges <= 253 && march_hist_fits(8, n_edges) &&
-                         (long long)nx * ny < (1LL << 28);
-  if (many_rois) IFE_TRY(ctx->ws.packed.reserve(ctx, n * sizeof(unsigned long long)));
-  const StencilCoef S = make_stencil_coef(spacing);
-  int box[6];         // only in-mask voxels (inside some ROI, when there are ROIs) are binned
-  bool have_box;
-  IFE_TRY(compute_support_box(ctx, d_mask, nx, ny, nz, rois, n_roi, box, &have_box));
-  MaskedPlan plan;
-  IFE_TRY(plan_masked(ctx, have_box, 0, d_img, d_mask, nx, ny, nz, rois, n_roi, &plan));
-  // no feature volume leaves this call, so with a crop the fused kernel runs on the crop too
-  // (its dims, its copy of the mask, the ROI list moved into its frame)
-  const int fx = plan.cropped ? plan.cdim[0] : nx, fy = plan.cropped ? plan.cdim[1] : ny,
-            fz = plan.cropped ? plan.cdim[2] : nz;
-  if (n_roi > 0) {
-    const std::vector<int> moved = plan.cropped ? rois_in_crop(plan, rois, n_roi) : std::vector<int>();
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws.rois.ptr, plan.cropped ? moved.data() : rois,
-                                      (size_t)n_roi * 6 * sizeof(int), cudaMemcpyHostToDevice, ctx->stream()));
-    if (plan.cropped) IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));   // `moved` is about to go
+  MaskedPlan plan;    // only in-mask voxels (inside some ROI, when there are ROIs) are binned
+  IFE_TRY(plan_masked(ctx, d_img, d_mask, nx, ny, nz, rois, n_roi, &plan));
+  {
+    std::vector<int> moved;
+    IFE_TRY(upload_rois(ctx, plan, rois, n_roi, d_rois, &moved));
+    if (!moved.empty()) IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));   // `moved` is about to go
   }
-  for (int s = 0; s < n_sigma && !(plan.have_box && plan.empty); ++s) {
-    float* blur = plan.cropped ? (float*)ctx->ws.crop_blur.ptr : (float*)ctx->ws.blur.ptr;
-    IFE_TRY(smooth_masked(ctx, plan, d_img, d_mask, blur, nx, ny, nz, spacing, sigmas[s], false));
-    FeatArgs A;
-    std::memset(&A, 0, sizeof(A));
-    A.vol = blur; A.mask_u8 = plan.mask;
-    A.nx = fx; A.ny = fy; A.nzb = fz; A.zb0 = 0; A.zb1 = fz;
-    A.hist.edges = (const float*)ctx->ws.edges.ptr + (size_t)s * 8 * n_edges;
-    A.hist.counts = d_counts + (size_t)s * 8 * nb;
-    A.hist.n_edges = n_edges;
-    A.hist.stride_roi = (long long)rows * nb;
-    if (many_rois) {
-      A.hist.packed = (unsigned long long*)ctx->ws.packed.ptr;
-      IFE_TRY(launch_features(ctx, 0, S, A, is_unit_spacing(spacing)));
-      ProfScope prof(ctx, K_OTHER);
-      roi_hist_packed_kernel<<<(unsigned)n_roi, 256, (size_t)8 * nb * sizeof(uint32_t), ctx->stream()>>>(
-          A.hist.packed, fx, fy, d_rois, nb, A.hist.counts, A.hist.stride_roi);
-      ctx->launches++;
-      IFE_CUDA_TRY(ctx, cudaGetLastError());
-    } else {
-      A.hist.rois = d_rois; A.hist.n_roi = n_roi;
-      IFE_TRY(launch_features(ctx, 0, S, A, is_unit_spacing(spacing)));
-    }
-  }
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(counts, d_counts, n_counts * sizeof(uint32_t),
-                                      cudaMemcpyDeviceToHost, ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  IFE_TRY(bin_masked_scan(ctx, plan, d_img, d_mask, nx, ny, nz, spacing, sigmas, n_sigma,
+                          (const float*)ctx->ws.edges.ptr, n_edges, d_rois, n_roi, d_counts));
+  return finish_out(ctx, counts, d_counts, n_counts, mem);
 }
 
 int ife_cuda_emphysema_histograms_batch(ife_cuda_ctx* ctx, int n_scans, const float* const* images,
@@ -1460,13 +1453,10 @@ int ife_cuda_emphysema_histograms_batch(ife_cuda_ctx* ctx, int n_scans, const fl
   IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int nx = dims[0], ny = dims[1], nz = dims[2];
   const size_t n = (size_t)nx * ny * nz;
-  for (int i = 0; i < n_scans; ++i)
+  for (int i = 0; i < n_scans; ++i) {
     if (!images[i] || !masks[i]) return fail(ctx, IFE_E_INVALID, "scan %d: null image or mask", i);
-  for (int r = 0; r < n_scans * n_roi; ++r) {
-    const int* b = rois + 6 * r;
-    if (b[0] < 0 || b[1] < 0 || b[2] < 0 || b[3] <= 0 || b[4] <= 0 || b[5] <= 0 ||
-        b[0] + b[3] > nx || b[1] + b[4] > ny || b[2] + b[5] > nz)
-      return fail(ctx, IFE_E_INVALID, "ROI %d is not inside the image", r);
+    if (check_rois(ctx, rois + (size_t)i * n_roi * 6, n_roi, dims) != IFE_OK)
+      return fail(ctx, IFE_E_INVALID, "scan %d: %s", i, ctx->error.c_str());
   }
   Workspace& ws = ctx->ws;
   IFE_TRY(reserve_smoothing(ctx, 2, nx, ny, nz));
@@ -1479,17 +1469,18 @@ int ife_cuda_emphysema_histograms_batch(ife_cuda_ctx* ctx, int n_scans, const fl
     IFE_TRY(mask_slot[k]->reserve(ctx, n));
   }
   if (ctx->host_image_i16) IFE_TRY(ws.in_i16.reserve(ctx, 2 * ((n + 3) & ~(size_t)3) * sizeof(short)));
-  const int rows = n_sigma * 8, nb = n_edges + 1, R = std::max(n_roi, 1);
-  const size_t n_counts = (size_t)R * rows * nb;
+  const int rows = n_sigma * 8, R = std::max(n_roi, 1);
+  const size_t n_counts = (size_t)R * rows * (n_edges + 1);
   IFE_TRY(ws.edges.reserve(ctx, (size_t)rows * n_edges * sizeof(float)));
   IFE_TRY(ws.counts.reserve(ctx, 2 * n_counts * sizeof(uint32_t)));
-  if (n_roi > 0) IFE_TRY(ws.rois.reserve(ctx, (size_t)n_scans * n_roi * 6 * sizeof(int)));
+  int* d_rois = nullptr;   // each scan's list, uploaded on the context's stream right before its kernels
+  if (n_roi > 0) {
+    IFE_TRY(ws.rois.reserve(ctx, (size_t)n_roi * 6 * sizeof(int)));
+    d_rois = (int*)ws.rois.ptr;
+  }
   cudaStream_t st = ctx->stream(), cp = ctx->copy_stream;
   IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ws.edges.ptr, edges, (size_t)rows * n_edges * sizeof(float),
                                     cudaMemcpyHostToDevice, st));
-  if (n_roi > 0)
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ws.rois.ptr, rois, (size_t)n_scans * n_roi * 6 * sizeof(int),
-                                      cudaMemcpyHostToDevice, st));
   const bool use_box = support_box_usable(ctx, (const uint8_t*)mask_slot[0]->ptr, nx, ny, nz) &&
                        support_box_usable(ctx, (const uint8_t*)mask_slot[1]->ptr, nx, ny, nz);
   // events[0..1]: upload of slot k done; events[2..3]: kernels reading slot k done
@@ -1508,7 +1499,6 @@ int ife_cuda_emphysema_histograms_batch(ife_cuda_ctx* ctx, int n_scans, const fl
     return IFE_OK;
   };
   IFE_TRY(upload(0));
-  const StencilCoef S = make_stencil_coef(spacing);
   std::vector<std::vector<int>> moved((size_t)n_scans);   // alive until the copies have run
   for (int i = 0; i < n_scans; ++i) {
     const int k = i & 1;
@@ -1522,27 +1512,9 @@ int ife_cuda_emphysema_histograms_batch(ife_cuda_ctx* ctx, int n_scans, const fl
     MaskedPlan plan;
     const int* scan_rois = n_roi > 0 ? rois + (size_t)i * n_roi * 6 : nullptr;
     IFE_TRY(plan_masked(ctx, use_box, k, d_img, d_mask, nx, ny, nz, scan_rois, n_roi, &plan));
-    const int fx = plan.cropped ? plan.cdim[0] : nx, fy = plan.cropped ? plan.cdim[1] : ny,
-              fz = plan.cropped ? plan.cdim[2] : nz;
-    if (plan.cropped && n_roi > 0) {   // this scan's ROIs in the frame of its crop
-      moved[i] = rois_in_crop(plan, scan_rois, n_roi);
-      IFE_CUDA_TRY(ctx, cudaMemcpyAsync((int*)ws.rois.ptr + (size_t)i * n_roi * 6, moved[i].data(),
-                                        (size_t)n_roi * 6 * sizeof(int), cudaMemcpyHostToDevice, st));
-    }
-    for (int s = 0; s < n_sigma && !(plan.have_box && plan.empty); ++s) {
-      float* blur = plan.cropped ? (float*)ws.crop_blur.ptr : (float*)ws.blur.ptr;
-      IFE_TRY(smooth_masked(ctx, plan, d_img, d_mask, blur, nx, ny, nz, spacing, sigmas[s], false));
-      FeatArgs A;
-      std::memset(&A, 0, sizeof(A));
-      A.vol = blur; A.mask_u8 = plan.mask;
-      A.nx = fx; A.ny = fy; A.nzb = fz; A.zb0 = 0; A.zb1 = fz;
-      A.hist.edges = (const float*)ws.edges.ptr + (size_t)s * 8 * n_edges;
-      A.hist.counts = d_counts + (size_t)s * 8 * nb;
-      A.hist.rois = n_roi > 0 ? (const int*)ws.rois.ptr + (size_t)i * n_roi * 6 : nullptr;
-      A.hist.n_roi = n_roi; A.hist.n_edges = n_edges;
-      A.hist.stride_roi = (long long)rows * nb;
-      IFE_TRY(launch_features(ctx, 0, S, A, is_unit_spacing(spacing)));
-    }
+    IFE_TRY(upload_rois(ctx, plan, scan_rois, n_roi, d_rois, &moved[i]));
+    IFE_TRY(bin_masked_scan(ctx, plan, d_img, d_mask, nx, ny, nz, spacing, sigmas, n_sigma,
+                            (const float*)ws.edges.ptr, n_edges, d_rois, n_roi, d_counts));
     IFE_CUDA_TRY(ctx, cudaEventRecord(ctx->events[2 + k], st));
     IFE_CUDA_TRY(ctx, cudaMemcpyAsync(counts + (size_t)i * n_counts, d_counts, n_counts * sizeof(uint32_t),
                                       cudaMemcpyDeviceToHost, st));
@@ -1565,11 +1537,8 @@ int ife_cuda_histogram(ife_cuda_ctx* ctx, const float* values, size_t n, const f
   IFE_TRY(ctx->ws.edges.reserve(ctx, n_edges * sizeof(float)));
   IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws.edges.ptr, edges, n_edges * sizeof(float),
                                     cudaMemcpyHostToDevice, ctx->stream()));
-  uint32_t* d_counts = counts;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.counts.reserve(ctx, (n_edges + 1) * sizeof(uint32_t)));
-    d_counts = (uint32_t*)ctx->ws.counts.ptr;
-  }
+  uint32_t* d_counts;
+  IFE_TRY(stage_out(ctx, ctx->ws.counts, counts, n_edges + 1, mem, &d_counts));
   IFE_CUDA_TRY(ctx, cudaMemsetAsync(d_counts, 0, (n_edges + 1) * sizeof(uint32_t), ctx->stream()));
   if (n > 0) {
     const unsigned grid = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)ctx->sm_count * 16);
@@ -1578,12 +1547,7 @@ int ife_cuda_histogram(ife_cuda_ctx* ctx, const float* values, size_t n, const f
     ctx->launches++;
     IFE_CUDA_TRY(ctx, cudaGetLastError());
   }
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(counts, d_counts, (n_edges + 1) * sizeof(uint32_t),
-                                      cudaMemcpyDeviceToHost, ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, counts, d_counts, n_edges + 1, mem);
 }
 
 int ife_cuda_intensity_roi_histograms(ife_cuda_ctx* ctx, const float* image, const uint8_t* mask,
@@ -1599,12 +1563,7 @@ int ife_cuda_intensity_roi_histograms(ife_cuda_ctx* ctx, const float* image, con
   IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int nx = dims[0], ny = dims[1], nz = dims[2];
   const size_t n = (size_t)nx * ny * nz;
-  for (int r = 0; r < n_roi; ++r) {
-    const int* b = rois + 6 * r;
-    if (b[0] < 0 || b[1] < 0 || b[2] < 0 || b[3] <= 0 || b[4] <= 0 || b[5] <= 0 ||
-        b[0] + b[3] > nx || b[1] + b[4] > ny || b[2] + b[5] > nz)
-      return fail(ctx, IFE_E_INVALID, "ROI %d is not inside the image", r);
-  }
+  IFE_TRY(check_rois(ctx, rois, n_roi, dims));
   const size_t smem = n_edges * sizeof(float) + (n_edges + 1) * sizeof(uint32_t);
   if (smem > 48 * 1024) return fail(ctx, IFE_E_INVALID, "too many histogram edges (%d)", n_edges);
   const float* d_img;
@@ -1618,11 +1577,8 @@ int ife_cuda_intensity_roi_histograms(ife_cuda_ctx* ctx, const float* image, con
   IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws.rois.ptr, rois, (size_t)n_roi * 6 * sizeof(int),
                                     cudaMemcpyHostToDevice, ctx->stream()));
   const size_t n_counts = (size_t)n_roi * (n_edges + 1);
-  uint32_t* d_counts = counts;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.counts.reserve(ctx, n_counts * sizeof(uint32_t)));
-    d_counts = (uint32_t*)ctx->ws.counts.ptr;
-  }
+  uint32_t* d_counts;
+  IFE_TRY(stage_out(ctx, ctx->ws.counts, counts, n_counts, mem, &d_counts));
   {
     ProfScope prof(ctx, K_OTHER);
     roi_intensity_hist_kernel<<<(unsigned)n_roi, 256, smem, ctx->stream()>>>(
@@ -1630,12 +1586,7 @@ int ife_cuda_intensity_roi_histograms(ife_cuda_ctx* ctx, const float* image, con
     ctx->launches++;
     IFE_CUDA_TRY(ctx, cudaGetLastError());
   }
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(counts, d_counts, n_counts * sizeof(uint32_t),
-                                      cudaMemcpyDeviceToHost, ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, counts, d_counts, n_counts, mem);
 }
 
 int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_bytes, const int dims[3],
@@ -1668,11 +1619,8 @@ int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_byt
   IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const uint8_t* d_in;
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, static_cast<const uint8_t*>(in), n_in * elem_bytes, mem, &d_in));
-  void* d_out = out;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, n_out * elem_bytes));
-    d_out = ctx->ws.out[0].ptr;
-  }
+  uint8_t* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], static_cast<uint8_t*>(out), n_out * elem_bytes, mem, &d_out));
   ResampleArgs A;
   std::memset(&A, 0, sizeof(A));
   A.in = d_in;
@@ -1704,11 +1652,7 @@ int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_byt
     ctx->launches++;
     IFE_CUDA_TRY(ctx, cudaGetLastError());
   }
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, n_out * elem_bytes, cudaMemcpyDeviceToHost, ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, static_cast<uint8_t*>(out), d_out, n_out * elem_bytes, mem);
 }
 
 // In-place device sort of n floats at d_data (csrc/radix_sort.cuh): 8 passes of count / scan / scatter
@@ -1745,11 +1689,7 @@ int ife_cuda_sort_f32(ife_cuda_ctx* ctx, float* data, size_t n, int mem) {
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, (const float*)data, n, mem, &d_in_c));
   float* d_in = const_cast<float*>(d_in_c);
   IFE_TRY(radix_sort_device(ctx, d_in, n));
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(data, d_in, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, data, d_in, n, mem);
 }
 
 // The compaction sink of the bin-edge determination: features on the device, only the sampled
@@ -1815,11 +1755,8 @@ int ife_cuda_emphysema_feature_samples(ife_cuda_ctx* ctx, const float* image, co
   IFE_TRY(reserve_smoothing(ctx, 2, nx, ny, nz));
   IFE_TRY(ctx->ws.blur.reserve(ctx, n * sizeof(float)));
   IFE_TRY(ctx->ws.out[0].reserve(ctx, 8 * n * sizeof(float)));
-  int box[6];
-  bool have_box;
-  IFE_TRY(compute_support_box(ctx, d_mask, nx, ny, nz, nullptr, 0, box, &have_box));
   MaskedPlan plan;
-  IFE_TRY(plan_masked(ctx, have_box, 0, d_img, d_mask, nx, ny, nz, nullptr, 0, &plan));
+  IFE_TRY(plan_masked(ctx, d_img, d_mask, nx, ny, nz, nullptr, 0, &plan));
   const size_t rows_bytes = (size_t)8 * n_sel * sizeof(float);
   float* d_rows = out;
   if (mem == IFE_MEM_HOST) {
@@ -1864,20 +1801,12 @@ int ife_cuda_eigen_features_batch(ife_cuda_ctx* ctx, const float* A6, float* out
   IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const float* d_in;
   IFE_TRY(stage_in(ctx, ctx->ws.in_img, A6, 6 * n, mem, &d_in));
-  float* d_out = out6;
-  if (mem == IFE_MEM_HOST) {
-    IFE_TRY(ctx->ws.out[0].reserve(ctx, 6 * n * sizeof(float)));
-    d_out = (float*)ctx->ws.out[0].ptr;
-  }
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out6, 6 * n, mem, &d_out));
   eigen_features_batch_lean_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream()>>>(d_in, d_out, n);
   ctx->launches++;
   IFE_CUDA_TRY(ctx, cudaGetLastError());
-  if (mem == IFE_MEM_HOST) {
-    IFE_CUDA_TRY(ctx, cudaMemcpyAsync(out6, d_out, 6 * n * sizeof(float), cudaMemcpyDeviceToHost,
-                                      ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
-  return IFE_OK;
+  return finish_out(ctx, out6, d_out, 6 * n, mem);
 }
 
 }  // extern "C"

@@ -149,12 +149,7 @@ static int slab_compute(ife_cuda_ctx* ctx, const float* bimg, const uint8_t* bma
     IFE_TRY(ws.edges.reserve(ctx, (size_t)rows * n_edges * sizeof(float)));
     IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ws.edges.ptr, edges, (size_t)rows * n_edges * sizeof(float),
                                       cudaMemcpyHostToDevice, st));
-    if (mem == IFE_MEM_HOST) {
-      IFE_TRY(ws.counts.reserve(ctx, (size_t)rows * nb * sizeof(uint32_t)));
-      d_counts = (uint32_t*)ws.counts.ptr;
-    } else {
-      d_counts = counts;
-    }
+    IFE_TRY(stage_out(ctx, ws.counts, counts, (size_t)rows * nb, mem, &d_counts));
     IFE_CUDA_TRY(ctx, cudaMemsetAsync(d_counts, 0, (size_t)rows * nb * sizeof(uint32_t), st));
   }
   if (d_counts_out) *d_counts_out = d_counts;
@@ -242,12 +237,9 @@ int ife_cuda_slab_emphysema_features_local(ife_cuda_ctx* ctx, const float* image
   IFE_TRY(slab_compute(ctx, d_img, d_mask, ext_z0, ext_z0 + ext_nz, own_z0, own_z0 + own_nz, out,
                        global_dims, spacing, sigmas, n_sigma, edges, n_edges, counts, halo_factor, mem,
                        &d_counts));
-  if (mem == IFE_MEM_HOST) {
-    if (edges)
-      IFE_CUDA_TRY(ctx, cudaMemcpyAsync(counts, d_counts, (size_t)n_sigma * 8 * (n_edges + 1) * sizeof(uint32_t),
-                                        cudaMemcpyDeviceToHost, ctx->stream()));
-    IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
-  }
+  // the wait also covers the per-scale copies of `out` that slab_compute enqueued
+  if (edges) return finish_out(ctx, counts, d_counts, (size_t)n_sigma * 8 * (n_edges + 1), mem);
+  if (mem == IFE_MEM_HOST) IFE_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream()));
   return IFE_OK;
 }
 
