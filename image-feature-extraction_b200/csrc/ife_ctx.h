@@ -70,7 +70,7 @@ struct ife_cuda_ctx {
   bool use_march4 = true;  // fused feature kernel with four voxels per thread where the layout allows (option "march4")
   bool host_image_i16 = false;   // host image pointers of the ife_cuda_emphysema_* calls are int16 (option "host_image_i16")
   bool use_box = true;     // masked paths smooth only the mask's support box (option "support_box")
-  int* box_host = nullptr; // pinned: the mask extents come back here once per call
+  int* box_host = nullptr; // pinned: the mask extents (or an expected distance's sums) come back here once per call
   bool overlap_scales = false;   // option "overlap_scales": features of scale s run beside the passes of scale s+1
   std::string error;
   ife::Workspace ws;

@@ -20,6 +20,7 @@
 
 #include <cuda_runtime.h>
 
+#include "distance_map.cuh"
 #include "eigen_features.cuh"
 #include "features_march.cuh"
 #include "features_march4.cuh"
@@ -1653,6 +1654,123 @@ int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_byt
     IFE_CUDA_TRY(ctx, cudaGetLastError());
   }
   return finish_out(ctx, static_cast<uint8_t*>(out), d_out, n_out * elem_bytes, mem);
+}
+
+// The three passes of a signed distance map (csrc/distance_map.cuh) on the context's stream.  With
+// A.partial set the z pass sums the weighted map into per-block partials instead of writing it.
+static int signed_distance_passes(ife_cuda_ctx* ctx, SdmArgs& A) {
+  const size_t n = (size_t)A.nx * A.ny * A.nz;
+  IFE_TRY(ctx->ws.a0.reserve(ctx, n * sizeof(int16_t)));
+  IFE_TRY(ctx->ws.a1.reserve(ctx, n * sizeof(uint32_t)));
+  IFE_TRY(ctx->ws.b0.reserve(ctx, n * sizeof(unsigned long long)));
+  A.gx = (int16_t*)ctx->ws.a0.ptr;
+  A.gxy = (uint32_t*)ctx->ws.a1.ptr;
+  A.stack = ctx->ws.b0.ptr;
+  cudaStream_t st = ctx->stream();
+  const unsigned rows = (unsigned)(((size_t)A.ny * A.nz + kSdmRowsPerBlock - 1) / kSdmRowsPerBlock);
+  const unsigned lines_y = (unsigned)(((size_t)A.nx * A.nz + kSdmLineThreads - 1) / kSdmLineThreads);
+  const unsigned lines_z = (unsigned)(((size_t)A.nx * A.ny + kSdmLineThreads - 1) / kSdmLineThreads);
+  {
+    ProfScope prof(ctx, K_OTHER);
+    sdm_pass_x<<<rows, 32 * kSdmRowsPerBlock, 0, st>>>(A);
+  }
+  {
+    ProfScope prof(ctx, K_OTHER);
+    sdm_pass_line<false, false><<<lines_y, kSdmLineThreads, 0, st>>>(A);
+  }
+  {
+    ProfScope prof(ctx, K_OTHER);
+    if (A.partial) sdm_pass_line<true, true><<<lines_z, kSdmLineThreads, 0, st>>>(A);
+    else sdm_pass_line<true, false><<<lines_z, kSdmLineThreads, 0, st>>>(A);
+  }
+  ctx->launches += 3;
+  IFE_CUDA_TRY(ctx, cudaGetLastError());
+  return IFE_OK;
+}
+
+// Arguments shared by the two distance entry points.
+static int check_distance_args(ife_cuda_ctx* ctx, const int dims[3], const double spacing[3], int flags, int allowed) {
+  if (flags & ~allowed) return fail(ctx, IFE_E_INVALID, "unknown flag bits 0x%x", flags & ~allowed);
+  IFE_TRY(check_dims(ctx, dims, spacing));
+  for (int d = 0; d < 3; ++d) {
+    if (!std::isfinite(spacing[d])) return fail(ctx, IFE_E_INVALID, "spacing[%d] is not finite", d);
+    if (dims[d] > kSdmMaxAxis)
+      return fail(ctx, IFE_E_INVALID, "dims[%d] = %d: a distance map takes axes of up to %d voxels", d, dims[d], kSdmMaxAxis);
+  }
+  return IFE_OK;
+}
+
+static SdmArgs distance_args(const int dims[3], const double spacing[3], const uint8_t* d_mask, int flags) {
+  SdmArgs A;
+  std::memset(&A, 0, sizeof(A));
+  A.nx = dims[0];
+  A.ny = dims[1];
+  A.nz = dims[2];
+  for (int d = 0; d < 3; ++d) A.s[d] = spacing[d];
+  A.mask = d_mask;
+  A.inside_positive = (flags & IFE_SDM_INSIDE_POSITIVE) != 0;
+  A.squared = (flags & IFE_SDM_SQUARED) != 0;
+  return A;
+}
+
+int ife_cuda_signed_distance_map(ife_cuda_ctx* ctx, const uint8_t* mask, float* out, const int dims[3],
+                                 const double spacing[3], int flags, int mem) {
+  if (!ctx) return IFE_E_INVALID;
+  if (!mask || !out) return fail(ctx, IFE_E_INVALID, "null pointer argument");
+  IFE_TRY(check_distance_args(ctx, dims, spacing, flags, IFE_SDM_INSIDE_POSITIVE | IFE_SDM_SQUARED));
+  const size_t n = (size_t)dims[0] * dims[1] * dims[2];
+  IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const uint8_t* d_mask;
+  IFE_TRY(stage_in(ctx, ctx->ws.in_mask, mask, n, mem, &d_mask));
+  float* d_out;
+  IFE_TRY(stage_out(ctx, ctx->ws.out[0], out, n, mem, &d_out));
+  SdmArgs A = distance_args(dims, spacing, d_mask, flags);
+  A.out = d_out;
+  IFE_TRY(signed_distance_passes(ctx, A));
+  return finish_out(ctx, out, d_out, n, mem);
+}
+
+int ife_cuda_expected_signed_distance(ife_cuda_ctx* ctx, const uint8_t* center, const float* weight,
+                                      const uint8_t* region, const int dims[3], const double spacing[3],
+                                      int flags, double* result, int mem) {
+  if (!ctx) return IFE_E_INVALID;
+  if (!center || !weight || !result) return fail(ctx, IFE_E_INVALID, "null pointer argument");
+  IFE_TRY(check_distance_args(ctx, dims, spacing, flags, IFE_SDM_INSIDE_POSITIVE));
+  const size_t n = (size_t)dims[0] * dims[1] * dims[2];
+  IFE_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const uint8_t *d_center, *d_region;
+  const float* d_weight;
+  IFE_TRY(stage_in(ctx, ctx->ws.in_mask, center, n, mem, &d_center));
+  IFE_TRY(stage_in(ctx, ctx->ws.in_img, weight, n, mem, &d_weight));
+  IFE_TRY(stage_in(ctx, ctx->ws.out[0], region, n, mem, &d_region));   // this call writes no volume
+  SdmArgs A = distance_args(dims, spacing, d_center, flags);
+  A.weight = d_weight;
+  A.region = d_region;
+  // the z pass's per-block partials and their sum go where the x pass's output was
+  const int n_blocks = (int)(((size_t)dims[0] * dims[1] + kSdmLineThreads - 1) / kSdmLineThreads);
+  IFE_TRY(ctx->ws.a0.reserve(ctx, std::max(n * sizeof(int16_t), (n_blocks + 1) * sizeof(SdmPartial))));
+  SdmPartial* partial = (SdmPartial*)ctx->ws.a0.ptr;
+  A.partial = partial;
+  IFE_TRY(signed_distance_passes(ctx, A));
+  if (!ctx->box_host)
+    IFE_CUDA_TRY(ctx, cudaHostAlloc((void**)&ctx->box_host, 12 * sizeof(int), cudaHostAllocDefault));
+  static_assert(sizeof(SdmPartial) <= 12 * sizeof(int), "the sums come back through box_host");
+  cudaStream_t st = ctx->stream();
+  {
+    ProfScope prof(ctx, K_OTHER);
+    sdm_reduce_partials<<<1, kSdmReduceThreads, 0, st>>>(partial, n_blocks, partial + n_blocks);
+    ctx->launches++;
+    IFE_CUDA_TRY(ctx, cudaGetLastError());
+  }
+  IFE_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->box_host, partial + n_blocks, sizeof(SdmPartial), cudaMemcpyDeviceToHost, st));
+  IFE_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  SdmPartial S;
+  std::memcpy(&S, ctx->box_host, sizeof(S));
+  if (S.no_site) return fail(ctx, IFE_E_INVALID, "the center mask has no contour voxel");
+  if (S.bad_weight) return fail(ctx, IFE_E_INVALID, "%d weights are negative or not finite", S.bad_weight);
+  if (!(S.sw > 0.0)) return fail(ctx, IFE_E_INVALID, "the weights sum to %g", S.sw);
+  *result = S.swd / S.sw;
+  return IFE_OK;
 }
 
 // In-place device sort of n floats at d_data (csrc/radix_sort.cuh): 8 passes of count / scan / scatter

@@ -17,6 +17,7 @@ HEADER_PATH = os.path.normpath(os.path.join(_HERE, "..", "include", "ife_cuda.h"
 
 MEM_HOST, MEM_DEVICE = 0, 1
 INTERP_LINEAR, INTERP_NEAREST = 0, 1
+SDM_INSIDE_POSITIVE, SDM_SQUARED = 1, 2
 ARITH_PLAIN, ARITH_FMA = 0, 1
 FDHF_TOOL_DY_BUG = 1
 NUM_FEATURES = 8
@@ -78,6 +79,8 @@ def load_library():
     L.ife_cuda_eigen_features_batch.argtypes = [vp, vp, vp, sz, i]
     L.ife_cuda_sort_f32.argtypes = [vp, vp, sz, i]
     L.ife_cuda_resample.argtypes = [vp, vp, vp, i, ip, dp, dp, i, d, ip, i]
+    L.ife_cuda_signed_distance_map.argtypes = [vp, vp, vp, ip, dp, i, i]
+    L.ife_cuda_expected_signed_distance.argtypes = [vp, vp, vp, vp, ip, dp, i, dp, i]
     L.ife_cuda_emphysema_feature_samples.argtypes = [vp, vp, vp, vp, vp, sz, ip, dp, dp, i, i, vp, C.POINTER(sz), i]
     L.ife_cuda_host_alloc.argtypes = [sz, C.POINTER(C.c_void_p)]
     L.ife_cuda_host_free.argtypes = [vp]
@@ -141,6 +144,10 @@ def _ptr(a):
     if isinstance(a, int):
         return C.c_void_p(a)
     return a.ctypes.data_as(C.c_void_p)
+
+
+def _sdm_flags(inside_positive, squared):
+    return (SDM_INSIDE_POSITIVE if inside_positive else 0) | (SDM_SQUARED if squared else 0)
 
 
 def _dims_of(vol):
@@ -371,6 +378,29 @@ class Context:
         self._check(self.L.ife_cuda_resample(self.h, _ptr(vol), _ptr(out), vol.dtype.itemsize, *args))
         return out
 
+    def signed_distance_map(self, mask, spacing=None, inside_positive=False, squared=False):
+        """(nz, ny, nx) mask (object = != 0) -> float32 signed Euclidean distance map (object negative
+        unless inside_positive; squared: the squared distance), in the units of spacing."""
+        mask = np.ascontiguousarray(mask, np.uint8)
+        out = np.empty(mask.shape, np.float32)
+        self._check(self.L.ife_cuda_signed_distance_map(self.h, _ptr(mask), _ptr(out), _i3(_dims_of(mask)),
+                                                        _d3(spacing), _sdm_flags(inside_positive, squared), MEM_HOST))
+        return out
+
+    def expected_distance(self, center, weight, region=None, spacing=None, inside_positive=False):
+        """sum(weight * signed distance to center's contour) / sum(weight) over region (or all voxels)
+        -> Python float."""
+        center = np.ascontiguousarray(center, np.uint8)
+        weight = np.ascontiguousarray(weight, np.float32)
+        r = None if region is None else np.ascontiguousarray(region, np.uint8)
+        if weight.shape != center.shape or (r is not None and r.shape != center.shape):
+            raise ValueError("center, weight and region must have one shape")
+        res = C.c_double()
+        self._check(self.L.ife_cuda_expected_signed_distance(
+            self.h, _ptr(center), _ptr(weight), _ptr(r), _i3(_dims_of(center)), _d3(spacing),
+            _sdm_flags(inside_positive, False), C.byref(res), MEM_HOST))
+        return res.value
+
     def eigen_features_batch(self, A6):
         A6 = np.ascontiguousarray(A6, np.float32).reshape(-1, 6)
         out = np.empty_like(A6)
@@ -412,6 +442,11 @@ class Context:
             self.h, _ptr(in_ptr), _ptr(out_ptr), elem_bytes, _i3(dims), _d3(spacing), _d3(out_spacing),
             INTERP_NEAREST if nearest else INTERP_LINEAR, float(default), od, MEM_DEVICE))
         return tuple(int(v) for v in od)
+
+    def signed_distance_map_dev(self, mask_ptr, out_ptr, dims, spacing=None, inside_positive=False, squared=False):
+        """Device-pointer signed distance map (uint8 in, float32 out), enqueued on the context's stream."""
+        self._check(self.L.ife_cuda_signed_distance_map(self.h, _ptr(mask_ptr), _ptr(out_ptr), _i3(dims), _d3(spacing),
+                                                        _sdm_flags(inside_positive, squared), MEM_DEVICE))
 
     def hessian_eigen_features_dev(self, img_ptr, mask_ptr, out_ptr, dims, sigma, spacing=None,
                                    flags=0):

@@ -264,6 +264,42 @@ int ife_cuda_resample(ife_cuda_ctx* ctx, const void* in, void* out, int elem_byt
                       const int dims[3], const double spacing[3], const double out_spacing[3],
                       int interp, double default_value, int out_dims[3], int mem);
 
+/* Signed Euclidean distance map of a mask: itk::SignedMaurerDistanceMapImageFilter as recalled (the
+ * reference's include/ife/Statistics/ExpectedDistanceFromCenterToInterestPoint.h builds on it; DESIGN.md
+ * "Signed distance maps" restates the semantics and what is this project's choice).
+ *   object = mask != 0.  A contour voxel is an object voxel with a background voxel among its 26
+ *   neighbours inside the image; voxels outside the image are not background, so the image border is
+ *   no contour.
+ *   D(v) = min over contour voxels c of fl(fl(fl((dx*sx)^2) + fl((dy*sy)^2)) + fl((dz*sz)^2)),
+ *   d = v - c in voxels, each square fl(t * t) of t = fl(d * s), every operation one rounded double
+ *   operation in this order.
+ *   out = (float)sqrt(D) (double sqrt, one rounding to float); IFE_SDM_SQUARED: out = (float)D.
+ *   Sign: object voxels are negated (ITK's InsideIsPositive off); IFE_SDM_INSIDE_POSITIVE negates
+ *   background voxels instead.  Only non-zero values are negated, so contour voxels are +0.0f: the
+ *   zero level is the object's inner layer and a background voxel touching the object is at +spacing.
+ *   No contour voxel anywhere (an empty mask, or one that fills the image): every voxel is FLT_MAX
+ *   with its side's sign.
+ *   ITK's UseImageSpacing off is spacing {1, 1, 1}.
+ * mask and out have the layout and `mem` of every volume of this ABI.  IFE_E_INVALID for a null
+ * pointer, unknown flag bits, a non-positive or non-finite spacing, or an axis longer than 32767
+ * voxels. */
+#define IFE_SDM_INSIDE_POSITIVE 1
+#define IFE_SDM_SQUARED 2
+int ife_cuda_signed_distance_map(ife_cuda_ctx* ctx, const uint8_t* mask, float* out, const int dims[3],
+                                 const double spacing[3], int flags, int mem);
+
+/* Expected signed distance: E = sum w(v) * (double)out(v) / sum w(v) over the voxels with
+ * region != 0 (every voxel when region is NULL), where out is the signed, non-squared map of
+ * ife_cuda_signed_distance_map of `center` with the same flags (IFE_SDM_INSIDE_POSITIVE is the only
+ * one) and w the `weight` image (a probability map).  The map is never written: the last pass sums it
+ * in double in a fixed partition and order, so two calls return the same bits.  The result is a host
+ * scalar, so the call always waits for the context's stream, whatever `mem` says of the volumes.
+ * IFE_E_INVALID as ife_cuda_signed_distance_map, and when a weight that enters the sum is negative or
+ * not finite, when those weights sum to 0, or when `center` has no contour voxel. */
+int ife_cuda_expected_signed_distance(ife_cuda_ctx* ctx, const uint8_t* center, const float* weight,
+                                      const uint8_t* region, const int dims[3], const double spacing[3],
+                                      int flags, double* result, int mem);
+
 /* Ascending in-place sort of n floats: the `std::sort` of the feature samples in
  * tools/DetermineHistogramBinEdges_MultiScaleEigenvalueFeatures.cxx:282-283.  A radix sort of
  * this library's own (csrc/radix_sort.cuh: 4-bit digits, count / scan / stable scatter; no
